@@ -453,6 +453,64 @@ def run_large_config(args):
         print(json.dumps(ln), flush=True)
 
 
+DUMP_SAMPLE = 16384                 # values kept of every larger parameter tensor
+DUMP_LIMIT_BYTES = 64 * 2 ** 20
+
+
+def _state_tensors(nets):
+    return [t for n in nets.values() for t in list(n.parameters()) + list(n.buffers())]
+
+
+def restore_initial_state(eng, initial):
+    """Put the training state back where the seeded construction left it: weights and buffers from ``initial``,
+    Adam moments and step counters at zero, the optimiser-maintained 16-bit operand planes re-packed from the
+    restored weights.  The kernels accumulate with atomics, so two runs of the same build drift apart step by
+    step; a step taken from this state sees the same inputs in every run."""
+    torch.cuda.synchronize()
+    with torch.no_grad():
+        for t, s in zip(_state_tensors(eng.nets), initial):
+            t.copy_(s)
+        for opt in eng.opts.values():
+            for st in opt.state.values():
+                st["exp_avg"].zero_()
+                st["exp_avg_sq"].zero_()
+            for st in opt._dev.values():
+                st["step"].zero_()
+        cache = eng.knets.weight_cache()
+        for ent in list(cache.d.values()):
+            if ent.spec is not None:
+                ent.fill(ent.val)
+                cache.refreshed(ent, ent.ref())
+    torch.cuda.synchronize()
+
+
+def dump_outputs(out_dir, nets, losses):
+    """What one step of the timed path hands its caller, as .npy files, so that two builds can be compared output
+    for output: ``losses.npy`` (float32: the loss vector ``GraphedStep.download`` delivers, in ``trainer.LOSS_KEYS``
+    order), ``<net>.params.npy`` (float32: the network's parameters after the step's Adam update, in
+    ``named_parameters`` order, of a tensor with more than DUMP_SAMPLE values a fixed seeded sample of DUMP_SAMPLE)
+    and ``<net>.buffers.npy`` (float64: every buffer in full -- BatchNorm running statistics and counters,
+    spectral-norm vectors)."""
+    import numpy as np
+    arrays = {"losses": losses.detach().float().cpu().numpy()}
+    g = torch.Generator().manual_seed(0)
+    for name, net in nets.items():
+        parts = []
+        for p in net.parameters():
+            flat = p.detach().reshape(-1)
+            if flat.numel() > DUMP_SAMPLE:
+                flat = flat[torch.randint(flat.numel(), (DUMP_SAMPLE,), generator=g).to(flat.device)]
+            parts.append(flat.float().cpu())
+        arrays[name + ".params"] = torch.cat(parts).numpy()
+        arrays[name + ".buffers"] = torch.cat([b.detach().reshape(-1).double().cpu() for b in net.buffers()]).numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def _recorded(name):
     """a measurement recorded under profiles/ (with its provenance) that the bench line quotes"""
     try:
@@ -493,7 +551,15 @@ def main():
     ap.add_argument("--segmented", action="store_true",
                     help="three CUDA graphs with the gradient all-reduces issued eagerly between them "
                          "instead of one graph that contains them")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="train config: after the timed loops take one more step of the timed path, untimed, from the "
+                         "seeded initial state, and write what it returned (losses, updated parameters -- a seeded "
+                         "sample of the large tensors -- and buffers) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl in ("reference", "stock-cuda") or args.config != "train"):
+        ap.error("--dump-outputs applies to the train config of this repo's CUDA path")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -525,6 +591,7 @@ def main():
         grad_sync = trainer.GradSync(enabled=False)
     eng = StepEngine(p, device, use_graph=not args.no_graph, grad_sync=grad_sync, segmented=args.segmented)
     eng.overlap_io = not args.serial_io and not args.no_graph and not args.segmented
+    initial = [t.detach().clone() for t in _state_tensors(eng.nets)] if args.dump_outputs else None
 
     # warm-up (eager: builds caches, sets kernel attributes), then capture
     side = torch.cuda.Stream()
@@ -599,6 +666,16 @@ def main():
         print("[bench] device-timed again after the e2e loop: %.3f ms/step (first %.3f, e2e %.3f)" % (
             timed_loop(False) / args.steps, ms_dev / args.steps, ms_e2e / args.steps), file=sys.stderr, flush=True)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # one more step through the timed path (same graph, same input upload and loss read-back), untimed, from
+        # the seeded initial state; every rank takes it (the graph holds the gradient exchange)
+        restore_initial_state(eng, initial)
+        eng.upload()
+        eng.step()
+        eng.download()
+        torch.cuda.synchronize()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, eng.nets, eng.loss_dev)
     if launches_per_step is None:
         launches_per_step = (c1 - c0) / args.steps
 
