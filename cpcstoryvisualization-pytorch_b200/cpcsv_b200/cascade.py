@@ -58,7 +58,7 @@ class DownConvNode(ConvNode):
 
 class MaskConv:
     """conv3x3 (stride 1, pad 1, no bias) of a few-channel NCHW fp32 image (the 1-channel mask) as
-    im2col + one K = 64 GEMM; the mirror of the discriminators' first layer (nets.EncoderRunner)."""
+    im2col + one K = 64 GEMM; the mirror of the video encoder's first layer (video.VideoEncoderRunner)."""
 
     def __init__(self, tape, weight, name):
         self.tape, self.w, self.name = tape, weight, name

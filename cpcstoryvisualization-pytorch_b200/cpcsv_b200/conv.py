@@ -11,13 +11,9 @@ SURVEY.md Appendix A): output pixel (2y+a, 2x+b) is a 2x2 conv of the LOW-RES in
 taps (i, j) at offsets (i-1+a, j-1+b) and merged weights -- 16 instead of 36 MACs per
 low-res pixel and the up-sampled tensor is never materialised.
 """
-import os
 from .ops import GemmJob, View, BF16
 
 NUM_SMS = 148
-# weight-gradient jobs as cta_group::2 pairs (two 128-channel M tiles share the x tile): the single-CTA kernel is
-# bound by the L2 -> SM feed at 42 % tensor-pipe activity (profiles/r02_stress512_tensor_pipe_table.txt)
-WGRAD_PAIR = os.environ.get("CPCSV_WGRAD_PAIR", "1") != "0"
 
 
 def pixel_tile(N, H, W, rows):
@@ -105,7 +101,9 @@ def _wgrad_job(a_view, b_view, grid, taps, m_valid, npad, out, ldc, dtype=BF16, 
                    k_blocks=0, taps=taps, a=[a_view], b=[b_view], out=out, n_valid=npad,
                    block_n=block_n, n_tiles=n_tiles, m_valid=m_valid, splits=splits, ldc=ldc,
                    dtype=dtype, accumulate=accumulate,
-                   pair=WGRAD_PAIR and m_valid > 128 and block_n % 128 == 0)
+                   # cta_group::2 pairs (two 128-channel M tiles share the x tile): the single-CTA kernel is bound by
+                   # the L2 -> SM feed at 42 % tensor-pipe activity (profiles/r02_stress512_tensor_pipe_table.txt)
+                   pair=m_valid > 128 and block_n % 128 == 0)
 
 
 def _planes(ts, fn):

@@ -5,20 +5,12 @@ ONE ``torch.autograd.Function`` whose inputs are the activations plus every para
 Reference call sites: generator trunk ``model.py:379-407 / 445-470``; encoders
 ``model.py:498-514, 540-556, 582-598``; ``D_GET_LOGITS.forward`` ``model.py:86-97``.
 """
-import os as _os
-
 import torch
 
 from . import conv, engine, ops
 from .engine import T4, BnActNode, ConvNode, GemmNode, SpectralNorm, Tape, rup, _e
 
 _CACHE = engine.WeightCache()
-
-# Run the spectral-norm power iterations of a discriminator call on a side stream, ahead of the
-# activation chain (they depend on the weights only).  No measurable gain on B200 (23.3 ms either
-# way): off by default, one less layer of nested stream forks.
-SN_AHEAD = _os.environ.get("CPCSV_SN_AHEAD", "0") == "1"
-DIRECT_ENC0 = _os.environ.get("CPCSV_DIRECT_ENC0", "1") != "0"     # first discriminator layer as one direct kernel
 
 
 def weight_cache():
@@ -542,7 +534,7 @@ def _row_pad_map(rows, rows_pad, dev):
 
 # =============================================================================== D encoder
 class EncoderRunner:
-    """encode_img: conv4x4 s2 (im2col GEMM for the 1/3-channel image) -> LeakyReLU, then 3 x
+    """encode_img: conv4x4 s2 -> LeakyReLU (one direct kernel, csrc/enc0.cu), then 3 x
     [SN conv4x4 s2 -> BN -> LeakyReLU].  Input x [n, C, 64, 64] fp32 (any strides); output
     features [n, 8*ndf, 4, 4] fp32 as a channels-last view."""
 
@@ -564,7 +556,8 @@ class EncoderRunner:
         enc0 = self.D.encode_img[0]
         return enc0.weight_orig if self.sn0 else enc0.weight
 
-    def _pack0(self, kind):
+    def _pack0(self):
+        """layer-0 weight as the B operand of the data-gradient GEMM: [64, Co_pad] with row tap*Ci + c"""
         w = self._w0()
         Co, Ci = w.shape[0], w.shape[1]
         Cop = rup(Co, 64)
@@ -573,81 +566,40 @@ class EncoderRunner:
 
         def build():
             w2 = w.detach().permute(0, 2, 3, 1).reshape(Co, K).contiguous()     # [co, tap*Ci + c]
-            if kind == "fwd":
-                hi, lo = _e((Cop, 64), w.device, torch.bfloat16), _e((Cop, 64), w.device, torch.bfloat16)
-                ops.pack_matrix(w2, Cop, 64, K, K, 1, _row_pad_map(Co, Cop, w.device), hi, lo)
-                return [hi, lo]
             hi = _e((64, Cop), w.device, torch.bfloat16)                         # [k, co]
             ops.pack_matrix(w2, 64, Cop, Co, 1, K, _row_pad_map(K, 64, w.device), hi, None)
             return hi
-        return _CACHE.get((id(w), "enc0_" + kind, 2), w, build)
+        return _CACHE.get((id(w), "enc0_bwd", 2), w, build)
 
     def run_forward(self, x, *plist):
         D = self.D
+        n, Cin, H, W = x.shape
+        w0 = self._w0()
+        Cop = rup(w0.shape[0], 64)
+        if not (Cop <= 128 and Cin in (1, 3) and H % 4 == 0 and W % 64 == 0):
+            raise NotImplementedError(
+                "cpcsv_b200: the first discriminator layer (csrc/enc0.cu) takes at most 128 output channels "
+                "(DF_DIM <= 128) and 1- or 3-channel images with H %% 4 == 0 and W %% 64 == 0; got %d output "
+                "channels, %d x %d x %d images" % (w0.shape[0], Cin, H, W))
         _eval_bn_unsupported(D)
         enc = D.encode_img
         dev = x.device
-        n, Cin, H, W = x.shape
         tape = Tape(_CACHE, training=D.training, need_grad=self.need_grad, planes=2, dtype=ops.BF16)
         self.tape = tape
         self.x_shape = (n, Cin, H, W)
         xd = x.detach()
-        # The spectral-norm power iterations depend on the weights only: all of them run on a side
-        # stream while layer 0 (im2col + GEMM + activation) runs here, instead of sitting in front
-        # of every convolution of the chain.
         Ho, Wo = H // 2, W // 2
-        w0 = self._w0()
-        Cop = rup(w0.shape[0], 64)
         sns = [SpectralNorm(enc[idx].weight_u, enc[idx].weight_v) for idx in (2, 5, 8)]
         self.sn_first = SpectralNorm(enc[0].weight_u, enc[0].weight_v) if self.sn0 else None
-
-        def power_iterations():
-            a0 = self.sn_first.forward(w0, D.training, self.need_grad) if self.sn_first is not None else None
-            return a0, [sn.forward(enc[idx].weight_orig, D.training, self.need_grad)
-                        for sn, idx in zip(sns, (2, 5, 8))]
-
-        def im2col():
-            col = T4(n, Ho, Wo, 64)
-            col.hi = _e((n, Ho, Wo, 64), dev, torch.bfloat16)
-            col.lo = _e((n, Ho, Wo, 64), dev, torch.bfloat16)
-            ops.im2col_small(xd, 4, 2, 1, col.hi, col.lo, 64)
-            return col, self._pack0("fwd")
-
-        from . import streams
-        # layer 0 in ONE launch (csrc/enc0.cu: conv + 1/sigma + LeakyReLU + hi/lo planes) whenever its geometry allows;
-        # otherwise im2col -> K = 64 GEMM -> activation
-        self.direct0 = DIRECT_ENC0 and Cop <= 128 and Cin in (1, 3) and H % 4 == 0 and W % 64 == 0
-        if self.direct0:
-            # layer 0 only needs its own 1 / sigma: the power iterations of layers 2, 5, 8 (a chain of ~15 small
-            # kernels that depends on the weights only) can run beside it
-            alpha0 = self.sn_first.forward(w0, D.training, self.need_grad) if self.sn_first is not None else None
-            self.alpha0, self.x0 = alpha0, xd
-
-            def later_sigmas():
-                return [sn.forward(enc[idx].weight_orig, D.training, self.need_grad)
-                        for sn, idx in zip(sns, (2, 5, 8))]
-
-            def layer0():
-                a = T4(n, Ho, Wo, Cop)
-                a.hi = _e((n, Ho, Wo, Cop), dev, torch.bfloat16)
-                a.lo = _e((n, Ho, Wo, Cop), dev, torch.bfloat16)
-                ops.enc0_lrelu_fwd(xd, w0.detach(), alpha0, 0.2, a.hi, a.lo, Cop)
-                return a
-            alphas, a = streams.concurrently(later_sigmas, layer0, enabled=SN_AHEAD)
-            self.a0 = a
-            self.col = self.z0 = self.act0 = None
-        else:
-            (alpha0, alphas), (col, w0p) = streams.concurrently(power_iterations, im2col, enabled=SN_AHEAD)
-            self.col = col
-            self.alpha0 = alpha0
-            z0 = T4(n, Ho, Wo, Cop)
-            z0.f32 = _e((n, Ho, Wo, Cop), dev)
-            ops.conv_gemm(conv.gemm_nt([col.hi.view(-1, 64), col.lo.view(-1, 64)], w0p,
-                                       z0.f32.view(-1, Cop), alpha=alpha0))
-            self.z0 = z0
-            act0 = BnActNode(tape, z0, None, ops.ACT_LRELU, "enc0.act")
-            a = tape.add(act0)
-            self.act0 = act0
+        alpha0 = self.sn_first.forward(w0, D.training, self.need_grad) if self.sn_first is not None else None
+        self.alpha0, self.x0 = alpha0, xd
+        alphas = [sn.forward(enc[idx].weight_orig, D.training, self.need_grad) for sn, idx in zip(sns, (2, 5, 8))]
+        # layer 0 in ONE launch: conv + 1/sigma + LeakyReLU + hi/lo planes
+        a = T4(n, Ho, Wo, Cop)
+        a.hi = _e((n, Ho, Wo, Cop), dev, torch.bfloat16)
+        a.lo = _e((n, Ho, Wo, Cop), dev, torch.bfloat16)
+        ops.enc0_lrelu_fwd(xd, w0.detach(), alpha0, 0.2, a.hi, a.lo, Cop)
+        self.a0 = a
         self.layers = []
         for li, idx in enumerate((2, 5, 8)):
             cmod, bmod = enc[idx], enc[idx + 1]
@@ -662,10 +614,7 @@ class EncoderRunner:
         self.feat = a
         Cf = enc[8].weight_orig.shape[0]
         tape.finish_forward()
-        if self.col is not None:
-            self.col.lo = None
-        else:
-            self.a0.lo = None
+        self.a0.lo = None
         return a.f32.permute(0, 3, 1, 2)[:, :Cf]
 
     def run_backward(self, grads, needs):
@@ -685,18 +634,15 @@ class EncoderRunner:
         w0 = self._w0()
         Co, Ci = w0.shape[0], w0.shape[1]
         K = 16 * Ci
+        a0 = self.a0
+        a0.needs_grad = True
         col_hi = None
-        if self.direct0:
-            self.a0.needs_grad = True
-            if need_w:
-                # the im2col matrix the layer-0 weight gradient multiplies with: built on the side branch at the START
-                # of the backward pass (it only needs the input image), consumed there at the end
-                n, Cin, H, W = self.x_shape
-                col_hi = _e((n * (H // 2) * (W // 2), 64), dev, torch.bfloat16)
-                self.tape.aux.run(lambda: ops.im2col_small(self.x0, 4, 2, 1, col_hi, None, 64))
-        else:
-            self.z0.needs_grad = True
-            col_hi = self.col.hi.view(-1, 64)
+        if need_w:
+            # the im2col matrix the layer-0 weight gradient multiplies with: built on the side branch at the START
+            # of the backward pass (it only needs the input image), consumed there at the end
+            n, Cin, H, W = self.x_shape
+            col_hi = _e((n * (H // 2) * (W // 2), 64), dev, torch.bfloat16)
+            self.tape.aux.run(lambda: ops.im2col_small(self.x0, 4, 2, 1, col_hi, None, 64))
         for cn, bn, idx in reversed(self.layers):
             bn.backward(need_w)
             pg["encode_img.%d.weight" % (idx + 1)] = bn.dgamma
@@ -704,16 +650,10 @@ class EncoderRunner:
             cn.backward(need_w)
             pg["encode_img.%d.weight_orig" % idx] = cn.dW
         # layer 0
-        if self.direct0:
-            a0 = self.a0
-            dz0 = _e((a0.N, a0.H, a0.W, a0.C), dev, torch.bfloat16)
-            ops.lrelu_bwd16(a0.grad, a0.hi, 0.2, dz0)
-            a0.grad = None
-            Cop = a0.C
-        else:
-            self.act0.backward(False)
-            dz0 = self.z0.grad16                                    # [n, 32, 32, Cop] bf16
-            Cop = self.z0.C
+        dz0 = _e((a0.N, a0.H, a0.W, a0.C), dev, torch.bfloat16)
+        ops.lrelu_bwd16(a0.grad, a0.hi, 0.2, dz0)
+        a0.grad = None
+        Cop = a0.C
         dz0m = dz0.view(-1, Cop)
         if need_w:
             def wgrad0():
@@ -723,22 +663,19 @@ class EncoderRunner:
                 if self.sn_first is not None:
                     gw = self.sn_first.backward(gw, w0)
                 pg[self.names[0]] = gw
-            if self.direct0:
-                self.tape.aux.run(wgrad0, dz0)
-            else:
-                wgrad0()
+            self.tape.aux.run(wgrad0, dz0)
         dx = None
         if needs[0]:
             n, Cin, H, W = self.x_shape
             dcol = _e((dz0m.shape[0], 64), dev)
-            ops.conv_gemm(conv.gemm_nt([dz0m, None], [self._pack0("bwd"), None], dcol, alpha=self.alpha0))
+            ops.conv_gemm(conv.gemm_nt([dz0m, None], [self._pack0(), None], dcol, alpha=self.alpha0))
             dx = _e((n, Cin, H, W), dev)
             ops.col2im_small(dcol, n, Cin, H, W, 4, 2, 1, dx)
         out = [dx]
         for nme, need in zip(self.names, needs[1:]):
             out.append(pg.get(nme) if need else None)
         self.tape.release()
-        self.tape = self.layers = self.act0 = self.z0 = self.col = self.feat = self.a0 = self.x0 = None
+        self.tape = self.layers = self.feat = self.a0 = self.x0 = None
         return out
 
 
@@ -778,19 +715,11 @@ class LogitsRunner:
         x = T4(n, H, W, Cc)
         sn = SpectralNorm(seq[0].weight_u, seq[0].weight_v)
         self.sn3 = SpectralNorm(seq[3].weight_u, seq[3].weight_v)
-        w3 = seq[3].weight_orig
-
-        def power_iterations():      # weights only: off the activation chain (side stream)
-            return (sn.forward(seq[0].weight_orig, L.training, self.need_grad),
-                    self.sn3.forward(w3, L.training, self.need_grad))
-
-        def pack_input():
-            x.hi = _e((n, H, W, Cc), dev, torch.bfloat16)
-            x.lo = _e((n, H, W, Cc), dev, torch.bfloat16)
-            ops.pack_nchw(h_code.detach(), c_code.detach().contiguous().view(n, Ce), x.hi, x.lo, Cc)
-
-        from . import streams
-        (alpha, inv_sigma), _ = streams.concurrently(power_iterations, pack_input, enabled=SN_AHEAD)
+        alpha = sn.forward(seq[0].weight_orig, L.training, self.need_grad)
+        inv_sigma = self.sn3.forward(seq[3].weight_orig, L.training, self.need_grad)
+        x.hi = _e((n, H, W, Cc), dev, torch.bfloat16)
+        x.lo = _e((n, H, W, Cc), dev, torch.bfloat16)
+        ops.pack_nchw(h_code.detach(), c_code.detach().contiguous().view(n, Ce), x.hi, x.lo, Cc)
         self.x, self.Cf = x, Cf
         cn = ConvNode(tape, "s1", x, seq[0].weight_orig, "logits.conv", sn=sn, alpha=alpha, bn_stats=True)
         z = tape.add(cn)

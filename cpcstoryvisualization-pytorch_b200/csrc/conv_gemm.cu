@@ -18,8 +18,6 @@
 #include <cuda.h>
 #include <cudaTypedefs.h>
 
-#include <stdlib.h>
-
 #include <mutex>
 
 #include "common.h"
@@ -32,6 +30,13 @@ constexpr int kBlockM = 128;
 constexpr int kMaxStages = 8;
 constexpr int kAPlaneBytes = kBlockM * 128;  // 128 rows x 64 16-bit (mode 0) / 2 x [64 pix x 64 ch] (mode 1)
 constexpr int kSmemLimit = 227 * 1024;
+// Shared memory a SINGLE-PLANE job takes: 144 KB = 3 pipeline stages of a pair job.  The single-plane jobs are the
+// backward pass and the no-grad forward; with the whole 227 KB (6 stages) a resident GEMM CTA leaves no room for any
+// other block that needs shared memory, and the optimiser's Adam + re-layout kernels (10-28 KB per block, issued
+// during the backward pass) queue up behind the last GEMM.  Measured (bench.py, two boxes): 227 KB 20.21 /
+// 20.59-20.61 ms per step; 160 KB 19.97 / 20.35; 144 KB 19.87-19.96; 128 KB 19.94-20.03 -- and no measurable change
+// of the GEMMs' own serial time (15.4-15.9 ms either way).
+constexpr int kSinglePlaneSmemLimit = 144 * 1024;
 constexpr int kBarrierBytes = 256;
 // Epilogue staging: each epilogue warp transposes its 32 rows x 32 columns through shared memory
 // so that global stores / red.adds cover whole 128 B row segments (4 rows per instruction)
@@ -515,37 +520,6 @@ static int make_map(CUtensorMap* tm, const cpcsv_view5_t& v, const uint32_t box[
   return 0;
 }
 
-// The cta_group::2 path is the default for fprop / dgrad jobs (CPCSV_PAIR=0 in the environment turns it
-// off).  Alone it is 0.79-0.87x the time on hi/lo-plane jobs and never slower (profiles/r01_sweep_pair.txt);
-// in the step 21.4-21.6 ms vs 22.1-22.3 ms with single CTAs (profiles/r02_pair_soak.log).  The intermittent
-// dead-lock of round 1 (6 of 12 runs) and of this round's first soaks (2 of 7 processes) was the TMEM
-// allocation handshake between the two CTAs of a cluster (kernel prologue above;
-// profiles/r02_pair_hang_rootcause.md); with the fix 32 of 32 processes x 150 whole-step graph replays ran
-// clean under the conditions that hung before (profiles/r02_pair_trace_after_fix.log).
-static bool pair_mode_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("CPCSV_PAIR");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
-// Shared memory a SINGLE-PLANE job takes (CPCSV_GEMM_SMEM_KB, 96..227; default 144 = 3 pipeline stages of a pair
-// job).  The single-plane jobs are the backward pass and the no-grad forward; with the whole 227 KB (6 stages) a
-// resident GEMM CTA leaves no room for any other block that needs shared memory, and the optimiser's Adam +
-// re-layout kernels (10-28 KB per block, issued during the backward pass) queue up behind the last GEMM.  Measured
-// (bench.py, two boxes): 227 KB 20.21 / 20.59-20.61 ms per step; 160 KB 19.97 / 20.35; 144 KB 19.87-19.96; 128 KB
-// 19.94-20.03 -- and no measurable change of the GEMMs' own serial time (15.4-15.9 ms either way).
-static int single_plane_smem_limit() {
-  static const int v = [] {
-    const char* e = getenv("CPCSV_GEMM_SMEM_KB");
-    int kb = e ? atoi(e) : 144;
-    if (kb < 96 || kb > 227) kb = 144;
-    return kb * 1024;
-  }();
-  return v;
-}
-
 int num_sms() {
   static int n = [] {
     int dev = 0, v = 0;
@@ -634,11 +608,17 @@ extern "C" int cpcsv_conv_gemm(const cpcsv_gemm_t* job, cpcsv_stream_t stream_) 
     CPCSV_REQUIRE(J.taps[i].out_off % 4 == 0, "conv_gemm: tap %d out_off alignment", i);
   }
   // CTA-pair mode (cta_group::2): jobs with at least two 128-row tiles whose B tile can be halved
-  // (fprop / dgrad: any block_n >= 32 in steps of 16; wgrad: whole 64-channel atoms per CTA)
+  // (fprop / dgrad: any block_n >= 32 in steps of 16; wgrad: whole 64-channel atoms per CTA).
+  // Alone a pair job is 0.79-0.87x the time of the single-CTA job on hi/lo-plane jobs and never slower
+  // (profiles/r01_sweep_pair.txt); in the step 21.4-21.6 ms vs 22.1-22.3 ms with single CTAs
+  // (profiles/r02_pair_soak.log).  The intermittent dead-lock of round 1 (6 of 12 runs) and of round 2's first
+  // soaks (2 of 7 processes) was the TMEM allocation handshake between the two CTAs of a cluster (kernel prologue
+  // above; profiles/r02_pair_hang_rootcause.md); with the fix 32 of 32 processes x 150 whole-step graph replays ran
+  // clean under the conditions that hung before (profiles/r02_pair_trace_after_fix.log).
   CPCSV_REQUIRE(J.cta_pair == 0 || (J.mode == 0 && J.block_n >= 32 && (J.block_n / 2) % 8 == 0) ||
                     (J.mode == 1 && (J.block_n / 2) % 64 == 0),
                 "conv_gemm: cta_pair needs block_n a multiple of 16 >= 32 (mode 0) or of 128 (mode 1)");
-  const bool pair = J.cta_pair != 0 && pair_mode_enabled() && P.m_tiles >= 2;
+  const bool pair = J.cta_pair != 0 && P.m_tiles >= 2;
   P.m_units = pair ? (P.m_tiles + 1) / 2 : P.m_tiles;
   const int64_t total = static_cast<int64_t>(P.groups) * P.splits * P.n_tiles * P.m_units;
   CPCSV_REQUIRE(total > 0 && total < (1ll << 31), "conv_gemm: tile count %lld", (long long)total);
@@ -647,7 +627,7 @@ extern "C" int cpcsv_conv_gemm(const cpcsv_gemm_t* job, cpcsv_stream_t stream_) 
                        pair ? 2 * kBlockM : kBlockM, static_cast<uint32_t>(J.block_n));
   P.b_plane_bytes = (pair ? J.block_n / 2 : J.block_n) * 128;
   P.stage_bytes = J.planes * (kAPlaneBytes + P.b_plane_bytes);
-  const int smem_limit = J.planes == 1 ? single_plane_smem_limit() : kSmemLimit;
+  const int smem_limit = J.planes == 1 ? kSinglePlaneSmemLimit : kSmemLimit;
   int stages = (smem_limit - 1024 - kBarrierBytes - kEpiBytes) / P.stage_bytes;
   if (stages > kMaxStages) stages = kMaxStages;
   CPCSV_REQUIRE(stages >= 2, "conv_gemm: tile does not fit shared memory");

@@ -99,3 +99,16 @@ def test_weight_cache_entries_die_with_their_parameter():
     get(b)
     assert len(built) == n + 1
     del key
+
+
+def test_first_discriminator_layer_past_its_kernel_limit_is_refused(monkeypatch):
+    """layer 0 of a discriminator is one direct kernel (csrc/enc0.cu) for at most 128 output channels:
+    DF_DIM 160 (padded to 192) raises instead of running some other path"""
+    import emulator
+    import harness
+    from oracle import params, presets
+    emulator.install(monkeypatch)
+    p = presets.get("tiny", DF_DIM=160)
+    D = harness.build_product(p, params.init_all(p, 0), torch.device("cpu"))["D_im"]
+    with pytest.raises(NotImplementedError, match="at most 128 output channels"):
+        D(torch.zeros(p["IM_BATCH"], 3, 64, 64))

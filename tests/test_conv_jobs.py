@@ -299,8 +299,8 @@ def test_temporal_conv_t3(dev, B, T, HW, Ci, Co):
 @pytest.mark.parametrize("geom,N,H,Ci,Co", [("s1", 6, 8, 128, 256), ("s1", 20, 4, 256, 384), ("s2", 5, 16, 128, 512),
                                              ("up", 3, 8, 384, 256), ("s1", 40, 8, 320, 256)])
 def test_wgrad_as_cta_pairs(dev, geom, N, H, Ci, Co):
-    """weight-gradient jobs with more than one 128-channel M tile run as cta_group::2 pairs (conv.WGRAD_PAIR):
-    even and odd numbers of M tiles, block_n 256 / 128 (and 64: no pair), split-K"""
+    """weight-gradient jobs with more than one 128-channel M tile and block_n a multiple of 128 run as
+    cta_group::2 pairs: even and odd numbers of M tiles, block_n 256 / 128 (and 64: no pair), split-K"""
     x = bf16r(rnd(N, Ci, H, H, seed=31, dev=dev))
     w = bf16r(rnd(Co, Ci, 4 if geom == "s2" else 3, 4 if geom == "s2" else 3, seed=32, dev=dev, scale=0.05))
     Ho = {"s1": H, "s2": H // 2, "up": 2 * H}[geom]
