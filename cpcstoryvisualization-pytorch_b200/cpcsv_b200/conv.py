@@ -118,16 +118,16 @@ def _plain_out_strides(out):
 
 
 # ------------------------------------------------------------------ k x k, stride 1
-def conv_s1_fwd(x_planes, w_planes, out, k=3, alpha=None, dtype=BF16):
+def conv_s1_fwd(x_planes, w_planes, out, k=3, alpha=None, dtype=BF16, splits=None):
     """out[N,H,W,Co] = conv(x[N,H,W,Ci], w), stride 1, pad k//2.  w_planes: packed kind 0
-    ``[k*k * Co_pad, Ci]``."""
+    ``[k*k * Co_pad, Ci]``.  ``splits``: split-K factor (None: pick_splits)."""
     N, H, W, Ci = x_planes[0].shape
     npad = out.shape[-1]
     pad = k // 2
     taps = [((0, kx - pad, 0, ky - pad), ((ky * k + kx) * npad, 0, 0, 0), 0)
             for ky in range(k) for kx in range(k)]
     return _fwd_job(_planes(x_planes, View.nhwc), _planes(w_planes, View.matrix), (N, H, W), 1,
-                    k * k, taps, Ci // 64, out, npad, _plain_out_strides(out), alpha, dtype=dtype)
+                    k * k, taps, Ci // 64, out, npad, _plain_out_strides(out), alpha, dtype=dtype, splits=splits)
 
 
 def conv_s1_dgrad(dy, wt, dx, k=3, alpha=None, accumulate=False):
@@ -198,7 +198,7 @@ def _s2_split(kk):
     return d % 2, d // 2
 
 
-def conv_s2_fwd(x_planes, w_planes, out, alpha=None, dtype=BF16):
+def conv_s2_fwd(x_planes, w_planes, out, alpha=None, dtype=BF16, splits=None):
     """out[N,H/2,W/2,Co] = conv4x4 s2 p1 (x[N,H,W,Ci]).  w_planes: kind 0 ``[16 * Co_pad, Ci]``."""
     N, H, W, Ci = x_planes[0].shape
     npad = out.shape[-1]
@@ -210,7 +210,7 @@ def conv_s2_fwd(x_planes, w_planes, out, alpha=None, dtype=BF16):
             taps.append(((wp * Ci, dw, hp, dh), ((ky * 4 + kx) * npad, 0, 0, 0), 0))
     return _fwd_job(_planes(x_planes, View.nhwc_parity), _planes(w_planes, View.matrix),
                     (N, H // 2, W // 2), 1, 16, taps, Ci // 64, out, npad, _plain_out_strides(out),
-                    alpha, dtype=dtype)
+                    alpha, dtype=dtype, splits=splits)
 
 
 def conv_s2_dgrad(dy, wt, dx, alpha=None):
@@ -252,7 +252,7 @@ def _rows_as_nhwc(t):
     return t.view(t.shape[0], 1, 1, t.shape[1])
 
 
-def gemm_nt(a_planes, b_planes, out, alpha=None, accumulate=False, dtype=BF16):
+def gemm_nt(a_planes, b_planes, out, alpha=None, accumulate=False, dtype=BF16, splits=None):
     """out[M, Npad] = a[M, K] @ b[Npad, K]^T  (K multiple of 64)."""
     M, K = a_planes[0].shape
     npad = out.shape[-1]
@@ -260,7 +260,7 @@ def gemm_nt(a_planes, b_planes, out, alpha=None, accumulate=False, dtype=BF16):
     taps = [((0, 0, 0, 0), (0, 0, 0, 0), 0)]
     av = [View.nhwc(_rows_as_nhwc(t)) for t in a_planes if t is not None]
     return _fwd_job(av, _planes(b_planes, View.matrix), (M, 1, 1), 1, 1, taps, K // 64, out, npad,
-                    (out.stride(0), 0, 0), alpha, accumulate, dtype=dtype)
+                    (out.stride(0), 0, 0), alpha, accumulate, dtype=dtype, splits=splits)
 
 
 def gemm_tn(a, b, out):
@@ -298,6 +298,34 @@ def conv_t3_fwd(x_planes, w_planes, out, alpha=None, dtype=BF16):
         jobs.append(_fwd_job([View.nhwc(t) for t in od], wv, (B, To, HW), 1, 2, taps, Ci // 64, out, npad,
                              _plain_out_strides(out), alpha, True, dtype=dtype, splits=1))
     return jobs
+
+
+def conv_t3s1_fwd(x_planes, w_planes, out, alpha=None, dtype=BF16, splits=None):
+    """Conv3d (3, 1, 1) stride 1 pad (1, 0, 0) of R(2+1)D-18 (torchvision Conv2Plus1D / R2Plus1dStem, the
+    reference's fid/residual2p1.py): out[B, T, HW, Co] = sum_kt x[B, t + kt - 1, HW, Ci] W_kt.  One job, three
+    taps; the zero fill of frames -1 and T is the temporal padding.  w_planes: kind 0 ``[3 * Co_pad, Ci]``."""
+    B, T, HW, Ci = x_planes[0].shape
+    npad = out.shape[-1]
+    assert tuple(out.shape[:3]) == (B, T, HW)
+    taps = [((0, 0, 0, kt - 1), (kt * npad, 0, 0, 0), 0) for kt in range(3)]
+    return _fwd_job(_planes(x_planes, View.nhwc), _planes(w_planes, View.matrix), (B, T, HW), 1, 3, taps,
+                    Ci // 64, out, npad, _plain_out_strides(out), alpha, dtype=dtype, splits=splits)
+
+
+def conv_p2_fwd(x_planes, w_planes, out, dtype=BF16, splits=None):
+    """Conv3d (1, 1, 1) stride (2, 2, 2) (the projected shortcut of a downsampling R(2+1)D-18 block):
+    out[B, To, H/2, W/2, Co] = x[B, 2 t, 2 y, 2 x, Ci] W, To = (T - 1) // 2 + 1.  The even frames of a [B, T, H,
+    W, C] tensor are no single uniform-stride batch dimension when B > 1, but ONE frame x[:, 2 t] is (batch stride
+    T*H*W*C, pixel pitch C): one single-tap parity-view job per output frame.  w_planes: kind 0 ``[Co_pad, Ci]``."""
+    B, T, H, W, Ci = x_planes[0].shape
+    To, npad = out.shape[1], out.shape[-1]
+    assert To == (T - 1) // 2 + 1 and tuple(out.shape[2:4]) == (H // 2, W // 2)
+    wv = _planes(w_planes, View.matrix)
+    taps = [((0, 0, 0, 0), (0, 0, 0, 0), 0)]
+    return [_fwd_job([View.nhwc_parity(p[:, 2 * t]) for p in x_planes if p is not None], wv, (B, H // 2, W // 2),
+                     1, 1, taps, Ci // 64, out[:, t], npad, _plain_out_strides(out[:, t]), dtype=dtype,
+                     splits=splits)
+            for t in range(To)]
 
 
 def conv_t3_dgrad(dy, wt, dx, alpha=None):

@@ -166,6 +166,21 @@ def bn_act_pack(x, scale, shift, act, mod=None, y=None, hi=None, lo=None, dtype=
         _ptr(y), ldy, _ptr(hi), _ptr(lo), ldp, dtype, _stream()), "cpcsv_bn_act_pack")
 
 
+def bn_add_act_pack(x, scale, shift, r, rscale, rshift, act, y=None, hi=None, lo=None, dtype=BF16):
+    """y = act(x*scale + shift + (r*rscale + rshift)); rscale / rshift None: identity shortcut (r as is)"""
+    rows, Cc, ld = _rows2d(x)
+    rr, rc, ldr = _rows2d(r)
+    assert (rr, rc) == (rows, Cc), (r.shape, x.shape)
+    ldy = y.stride(0) if y is not None else 0
+    ldp = hi.stride(0) if hi is not None else 0
+    if lo is not None:
+        assert lo.stride(0) == ldp
+    _lib.check(_lib.load().cpcsv_bn_add_act_pack(
+        _ptr(x, torch.float32), rows, Cc, ld, _ptr(scale, torch.float32), _ptr(shift, torch.float32),
+        _ptr(r, torch.float32), ldr, _ptr(rscale, torch.float32), _ptr(rshift, torch.float32), act,
+        _ptr(y, torch.float32), ldy, _ptr(hi), _ptr(lo), ldp, dtype, _stream()), "cpcsv_bn_add_act_pack")
+
+
 def bn_bwd_reduce(x, dy, scale, shift, mean, invstd, act, mod, sums):
     rows, Cc, ld = _rows2d(x)
     _lib.check(_lib.load().cpcsv_bn_bwd_reduce(

@@ -244,6 +244,54 @@ act_pack_kernel(const float* __restrict__ x, int64_t rows, int C, int64_t ldx,
   }
 }
 
+// ------------------------------------------------------------------------- residual epilogue
+// y = act(x*scale + shift + (r*rscale + rshift)): the last BatchNorm of a residual block, the BatchNorm of
+// its projected shortcut (kRS; identity shortcut: r as is), the add and the activation in one pass.
+template <bool kRS, bool kY, bool kHi, bool kLo>
+__global__ void __launch_bounds__(256)
+act_add_pack_kernel(const float* __restrict__ x, int64_t rows, int C, int64_t ldx,
+                    const float* __restrict__ scale, const float* __restrict__ shift,
+                    const float* __restrict__ r, int64_t ldr, const float* __restrict__ rscale,
+                    const float* __restrict__ rshift, int act, float* __restrict__ y, int64_t ldy,
+                    uint16_t* __restrict__ hi, uint16_t* __restrict__ lo, int64_t ldp, int dtype, int qpb,
+                    int rpb) {
+  const int ql = threadIdx.x % qpb, rl = threadIdx.x / qpb;
+  const int c = (blockIdx.x * qpb + ql) * 4;
+  if (c >= C) return;
+  float sc[4], sf[4], rsc[4] = {1.f, 1.f, 1.f, 1.f}, rsf[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    sc[j] = scale[c + j];
+    sf[j] = shift[c + j];
+    if (kRS) { rsc[j] = rscale[c + j]; rsf[j] = rshift[c + j]; }
+  }
+  const int64_t step = static_cast<int64_t>(gridDim.y) * rpb;
+  for (int64_t row = static_cast<int64_t>(blockIdx.y) * rpb + rl; row < rows; row += step) {
+    const float4 xv = *reinterpret_cast<const float4*>(x + row * ldx + c);
+    const float4 rv = *reinterpret_cast<const float4*>(r + row * ldr + c);
+    const float xs[4] = {xv.x, xv.y, xv.z, xv.w}, rs[4] = {rv.x, rv.y, rv.z, rv.w};
+    float v[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const float res = kRS ? fmaf(rs[j], rsc[j], rsf[j]) : rs[j];
+      v[j] = apply_act(fmaf(xs[j], sc[j], sf[j]) + res, act);
+    }
+    if (kY) *reinterpret_cast<float4*>(y + row * ldy + c) = make_float4(v[0], v[1], v[2], v[3]);
+    if (kHi) {
+      uint2 hv;
+      hv.x = pack2(v[0], v[1], dtype);
+      hv.y = pack2(v[2], v[3], dtype);
+      *reinterpret_cast<uint2*>(hi + row * ldp + c) = hv;
+      if (kLo) {
+        uint2 lv;
+        lv.x = pack2(v[0] - round16(v[0], dtype), v[1] - round16(v[1], dtype), dtype);
+        lv.y = pack2(v[2] - round16(v[2], dtype), v[3] - round16(v[3], dtype), dtype);
+        *reinterpret_cast<uint2*>(lo + row * ldp + c) = lv;
+      }
+    }
+  }
+}
+
 // ------------------------------------------------------------------------- backward
 struct ChanConst {
   float sc[4], sf[4], mean[4], invstd[4];
@@ -480,6 +528,41 @@ extern "C" int cpcsv_bn_norm_act_pack(const float* x, int64_t rows, int32_t C, i
   nb.C_valid = C_valid; nb.eps = eps; nb.momentum = momentum;
   return launch_act_pack(x, rows, C, ldx, nullptr, nullptr, act, mod, ldmod, y, ldy, hi, lo, ldp, dtype, nb,
                          STREAM(stream), "bn_norm_act_pack");
+}
+
+extern "C" int cpcsv_bn_add_act_pack(const float* x, int64_t rows, int32_t C, int64_t ldx, const float* scale,
+                                     const float* shift, const float* r, int64_t ldr, const float* rscale,
+                                     const float* rshift, int32_t act, float* y, int64_t ldy, void* hi, void* lo,
+                                     int64_t ldp, int32_t dtype, cpcsv_stream_t stream) {
+  CPCSV_REQUIRE(x && r && scale && shift && rows > 0 && C > 0 && C % 4 == 0 && ldx % 4 == 0 && ldr % 4 == 0,
+                "bn_add_act_pack: args");
+  CPCSV_REQUIRE(!rscale == !rshift, "bn_add_act_pack: rscale and rshift go together");
+  CPCSV_REQUIRE((!y || ldy % 4 == 0) && (!hi || ldp % 4 == 0), "bn_add_act_pack: pitches must be multiples of 4");
+  CPCSV_REQUIRE(hi || y, "bn_add_act_pack: no output");
+  CPCSV_REQUIRE(!lo || hi, "bn_add_act_pack: lo without hi");
+  const Tiling t = make_tiling(rows, C, 8, 4);
+  uint16_t* h = static_cast<uint16_t*>(hi);
+  uint16_t* l = static_cast<uint16_t*>(lo);
+#define LAUNCH(RS, Y, H, L)                                                                                   \
+  act_add_pack_kernel<RS, Y, H, L><<<t.grid, 256, 0, STREAM(stream)>>>(x, rows, C, ldx, scale, shift, r, ldr, \
+                                                                        rscale, rshift, act, y, ldy, h, l,    \
+                                                                        ldp, dtype, t.qpb, t.rpb)
+  const int key = (rscale ? 8 : 0) | (y ? 4 : 0) | (hi ? 2 : 0) | (lo ? 1 : 0);
+  switch (key) {
+    case 2: LAUNCH(false, false, true, false); break;
+    case 3: LAUNCH(false, false, true, true); break;
+    case 4: LAUNCH(false, true, false, false); break;
+    case 6: LAUNCH(false, true, true, false); break;
+    case 7: LAUNCH(false, true, true, true); break;
+    case 10: LAUNCH(true, false, true, false); break;
+    case 11: LAUNCH(true, false, true, true); break;
+    case 12: LAUNCH(true, true, false, false); break;
+    case 14: LAUNCH(true, true, true, false); break;
+    case 15: LAUNCH(true, true, true, true); break;
+    default: return fail(-1, "bn_add_act_pack: unsupported output combination %d", key);
+  }
+#undef LAUNCH
+  return launched("bn_add_act_pack");
 }
 
 extern "C" int cpcsv_bn_bwd_reduce(const float* x, const float* dy, int64_t rows, int32_t C,

@@ -755,6 +755,39 @@ class GANTrainer(object):
             self._logger.add_scalar("Evaluation/fid", fid_value, epoch)
         return vfid_value, fid_value
 
+    def calculate_fsd(self, netG, testloader, feature_net, real_stats=None, epoch=None, seed=0):
+        """Story-level Frechet distance (FSD) of generated test stories on the kernel path (cpcsv_b200.fsd):
+        R(2+1)D-18 features (``feature_net``, a ``fsd.StoryFeatureNet``) of the real ``images`` of every test
+        batch and of the stories ``netG.sample_videos`` generates for the same batch, whole batches per call,
+        with the generator in eval mode under no_grad.  ``real_stats``: a ``fsd.FeatureStats`` of the real
+        stories computed (or ``FeatureStats.load``-ed) before; the real images are then not run again.  The
+        generator's noise is drawn from a generator seeded with ``seed`` (the global RNG state is restored
+        afterwards), so the value is reproducible.  ``netG`` is left in train mode."""
+        from cpcsv_b200 import fsd
+        dev = next(netG.parameters()).device
+        text_dim = cfg.TEXT.DIMENSION
+        real = fsd.FeatureStats() if real_stats is None else None
+        fake = fsd.FeatureStats()
+        netG.eval()
+        try:
+            with torch.no_grad(), torch.random.fork_rng(devices=[dev] if dev.type == "cuda" else []):
+                torch.manual_seed(seed)
+                for batch in testloader:
+                    description = batch["description"].to(dev)
+                    st_content = description[:, :, :text_dim]
+                    st_motion = torch.cat((st_content, batch["labels"].to(dev)), 2)
+                    _, fake_stories, _, _, _, _, _ = netG.sample_videos(st_motion, st_content)
+                    fake.update(feature_net(fake_stories))
+                    if real is not None:
+                        real.update(feature_net(batch["images"].to(dev)))
+        finally:
+            netG.train()
+        real = real if real is not None else real_stats
+        value = fsd.frechet_distance(real.mu, real.sigma, fake.mu.to(real.mu.device), fake.sigma.to(real.mu.device))
+        if self._logger is not None:
+            self._logger.add_scalar("Evaluation/fsd", value, epoch)
+        return value
+
     GRAPH_WARMUP_STEPS = 3      # eager steps (optimiser state, weight caches, NCCL) before the capture
 
     def _shard_loader(self, loader):

@@ -152,6 +152,19 @@ int cpcsv_bn_norm_act_pack(const float* x, int64_t rows, int32_t C, int64_t ldx,
                            float* y, int64_t ldy, void* hi, void* lo, int64_t ldp, int32_t dtype,
                            cpcsv_stream_t stream);
 
+/* end of an R(2+1)D-18 BasicBlock in eval mode (torchvision.models.video.resnet.BasicBlock, which the
+ * reference's fid/residual2p1.py builds and fid/vfid_score.py runs for the story-level FID):
+ *   y = act(x*scale + shift + (r*rscale + rshift))
+ * x is the fp32 output of the block's last conv, r the shortcut [rows, C] (pitch ldr): the block input
+ * (rscale == rshift == NULL, identity shortcut) or the output of its (1,1,1) stride-2 projection conv
+ * (rscale / rshift: that branch's eval-mode BatchNorm).  scale / shift: the block's last BatchNorm.
+ * Writes any of fp32 y (the next block's identity shortcut), 16-bit hi, 16-bit lo; rows / pitches /
+ * channel padding as cpcsv_bn_act_pack (padding channels have zero scale, shift and residual). */
+int cpcsv_bn_add_act_pack(const float* x, int64_t rows, int32_t C, int64_t ldx, const float* scale,
+                          const float* shift, const float* r, int64_t ldr, const float* rscale,
+                          const float* rshift, int32_t act, float* y, int64_t ldy, void* hi, void* lo,
+                          int64_t ldp, int32_t dtype, cpcsv_stream_t stream);
+
 /* ------------------------------------------------------------------- layout / pack kernels */
 /* generated frames / image sheets for the PNG writers (miscc/utils.py:230-235 images_to_numpy,
  * inference.py:181-197): x [C, H, W] fp32 in [-1, 1] with element strides (sc, sh, sw) ->
