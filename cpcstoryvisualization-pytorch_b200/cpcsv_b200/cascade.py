@@ -5,125 +5,26 @@ ReLU), and the re-encoded features modulate the image trunk (``cascade_model.py:
 ``train_autoencoder`` (``cascade_model.py:528-540``) is the mask auto-encoder built from the same
 layers.  Every arithmetic step is one of the libcpcsv.so kernels the plain generator already uses:
 
-* downBlock conv = the 4x4 / stride-2 / pad-1 implicit GEMM of the discriminators with the 3x3
-  kernel embedded in the upper-left taps (same input coordinate ``2*o + k - 1``; the 4th row and
-  column of the packed weight are zero), so forward, dgrad and wgrad reuse the parity-view jobs;
+* downBlock conv = engine.ConvNode's ``s2k3`` geometry: the 4x4 / stride-2 / pad-1 implicit GEMM of the
+  discriminators with the 3x3 kernel embedded in the upper-left taps (same input coordinate
+  ``2*o + k - 1``; the 4th row and column of the packed weight are zero), so forward, dgrad and wgrad
+  reuse the parity-view jobs;
 * its bias is directly followed by a batch-statistics BatchNorm, which removes it from the
   output: it is not added at all, its gradient is identically zero, and only the BatchNorm
   running mean sees it (``running_mean += momentum * bias`` after the statistics kernel);
-* presample (1 input channel) = im2col'd K = 64 GEMM like the first discriminator layer.
+* presample (1 input channel) = im2col'd K = 64 GEMM (engine.Im2colNode).
 
 The intermediate activations the reference returns as ``latents`` (``cascade_model.py:441-445``)
 are outputs of the autograd Function; their incoming gradients (latent-MSE losses,
 ``trainer.py:369-376``) are injected into the tape's gradient slots.
 """
 import torch
-import torch.nn.functional as F
 
-from . import conv, ops
-from .engine import T4, BnActNode, ConvNode, StateOrder, Tape, rup, _e
-from .nets import _CACHE, TapeFn, TrunkRunner, _alias, _bn_tuple, _eval_needs_no_grad, _row_pad_map
+from . import ops
+from .engine import BnActNode, ConvNode, Im2colNode, StateOrder, Tape, rup
+from .nets import _CACHE, TapeFn, TrunkRunner, _alias, _bn_tuple, _eval_needs_no_grad
 
 BN_MOMENTUM = 0.1
-
-
-class DownConvNode(ConvNode):
-    """conv3x3 stride 2 pad 1 as the "s2" (4x4 stride 2 pad 1) geometry with zero 4th taps."""
-
-    def __init__(self, tape, x, weight, name):
-        super().__init__(tape, "s2", x, weight, name)
-
-    def _pack(self, kindcode, rows_pad, cols_pad, planes, dtype=ops.BF16):
-        w = self.w
-
-        def build():
-            w4 = F.pad(w.detach(), (0, 1, 0, 1)).contiguous()        # [Co, Ci, 4, 4], taps (3, .) / (., 3) zero
-            t16 = ops.TORCH16[dtype]
-            hi = _e((16 * rows_pad, cols_pad), w.device, t16)
-            lo = _e((16 * rows_pad, cols_pad), w.device, t16) if planes == 2 else None
-            ops.pack_conv_weight(w4, kindcode, rows_pad, cols_pad, hi, lo, dtype)
-            return [hi, lo]
-        # keyed on the 3x3 PARAMETER (the padded copy is a temporary whose id may be recycled)
-        return self.tape.cache.get((id(w), "down3x3", kindcode, planes, dtype), w, build)
-
-    def _wgrad(self, dz):
-        x = self.x
-        dev = dz.device
-        dwt = _e((16, self.Co_pad, self.Ci_pad), dev)
-        ops.conv_gemm(conv.conv_s2_wgrad(dz, x.hi, dwt))
-        g4 = _e((self.Co, self.Ci, 4, 4), dev)
-        ops.unpack_conv_wgrad(dwt, self.Co_pad * self.Ci_pad, self.Ci_pad, 0, None, g4)
-        self.dW = g4[:, :, :3, :3].contiguous()
-
-
-class MaskConv:
-    """conv3x3 (stride 1, pad 1, no bias) of a few-channel NCHW fp32 image (the 1-channel mask) as
-    im2col + one K = 64 GEMM; the mirror of the video encoder's first layer (video.VideoEncoderRunner)."""
-
-    def __init__(self, tape, weight, name):
-        self.tape, self.w, self.name = tape, weight, name
-        self.Co, self.Ci = weight.shape[0], weight.shape[1]
-        self.Cop = rup(self.Co, 64)
-        self.K = 9 * self.Ci
-        assert self.K <= 64, name
-        self.col = self.out = self.dW = None
-
-    def _pack(self, kind):
-        w, Co, Cop, K = self.w, self.Co, self.Cop, self.K
-        planes, dtype = self.tape.planes, self.tape.dtype
-
-        def build():
-            w2 = w.detach().permute(0, 2, 3, 1).reshape(Co, K).contiguous()      # [co, tap*Ci + c]
-            if kind == "fwd":
-                t16 = ops.TORCH16[dtype]
-                hi = _e((Cop, 64), w.device, t16)
-                lo = _e((Cop, 64), w.device, t16) if planes == 2 else None
-                ops.pack_matrix(w2, Cop, 64, K, K, 1, _row_pad_map(Co, Cop, w.device), hi, lo, dtype)
-                return [hi, lo]
-            hi = _e((64, Cop), w.device, torch.bfloat16)                          # [k, co]
-            ops.pack_matrix(w2, 64, Cop, Co, 1, K, _row_pad_map(K, 64, w.device), hi, None)
-            return hi
-        key = (id(w), "mask_" + kind, planes, dtype) if kind == "fwd" else (id(w), "mask_bwd", 1, ops.BF16)
-        return _CACHE.get(key, w, build)
-
-    def forward(self, x):
-        """x [n, Ci, H, W] fp32 (any strides) -> T4 with the fp32 conv output [n, H, W, Cop]"""
-        t = self.tape
-        n, Ci, H, W = x.shape
-        assert Ci == self.Ci
-        dev = x.device
-        t16 = ops.TORCH16[t.dtype]
-        col = T4(n, H, W, 64)
-        col.hi = _e((n, H, W, 64), dev, t16)
-        col.lo = _e((n, H, W, 64), dev, t16) if t.planes == 2 else None
-        ops.im2col_small(x.detach(), 3, 1, 1, col.hi, col.lo, 64, t.dtype)
-        z = T4(n, H, W, self.Cop)
-        z.f32 = _e((n, H, W, self.Cop), dev)
-        ops.conv_gemm(conv.gemm_nt([col.hi.view(-1, 64), col.lo.view(-1, 64) if col.lo is not None else None],
-                                   self._pack("fwd"), z.f32.view(-1, self.Cop), dtype=t.dtype))
-        col.lo = None
-        self.col, self.out, self.x_shape = col, z, (n, Ci, H, W)
-        return z
-
-    def backward(self, need_w, need_dx):
-        """consumes out.grad16; returns d(x) [n, Ci, H, W] fp32 or None"""
-        dz = self.out.grad16.view(-1, self.Cop)
-        dev = dz.device
-        if need_w:
-            def wgrad():
-                d = _e((self.Cop, 64), dev)
-                ops.conv_gemm(conv.gemm_tn(dz, self.col.hi.view(-1, 64), d))
-                self.dW = d[:self.Co, :self.K].reshape(self.Co, 3, 3, self.Ci).permute(0, 3, 1, 2).contiguous()
-            self.tape.aux.run(wgrad, dz)
-        dx = None
-        if need_dx:
-            n, Ci, H, W = self.x_shape
-            dcol = _e((dz.shape[0], 64), dev)
-            ops.conv_gemm(conv.gemm_nt([dz, None], [self._pack("bwd"), None], dcol))
-            dx = _e((n, Ci, H, W), dev)
-            ops.col2im_small(dcol, n, Ci, H, W, 3, 1, 1, dx)
-        self.out.grad16 = None
-        return dx
 
 
 class SegEncoder:
@@ -140,14 +41,14 @@ class SegEncoder:
     def forward(self, seg, want_f32=True):
         """seg [n, 1, 64, 64] fp32 -> activations (g_seg1 4x4, g_seg2 8x8, g_seg3 16x16, g_seg4 32x32)"""
         tape, G = self.tape, self.G
-        self.pre = MaskConv(tape, G.presample[0].weight, "presample")
-        z = self.pre.forward(seg)
+        self.pre = Im2colNode(tape, seg, G.presample[0].weight, "presample", 1, 1)
+        z = tape.add(self.pre)
         self.pre_bn = BnActNode(tape, z, _bn_tuple(G.presample[1]), ops.ACT_RELU, "presample.bn")
         a = tape.add(self.pre_bn)
         outs = []
         for i in range(1, 5):
             blk = getattr(G, "downsample%d_seg" % i)
-            cn = DownConvNode(tape, a, blk[0].weight, "downsample%d_seg" % i)
+            cn = ConvNode(tape, "s2k3", a, blk[0].weight, "downsample%d_seg" % i)
             zc = tape.add(cn)
             bn = BnActNode(tape, zc, _bn_tuple(blk[1]), ops.ACT_RELU, "downsample%d_seg.bn" % i,
                            want_f32=want_f32, pre_bias=blk[0].bias)
@@ -191,7 +92,7 @@ class SegEncoder:
 def _resolve(pg):
     """weight gradients produced on the aux branch are read from their nodes after the join"""
     for k, v in list(pg.items()):
-        if isinstance(v, (ConvNode, MaskConv)):
+        if isinstance(v, (ConvNode, Im2colNode)):
             pg[k] = v.dW
 
 

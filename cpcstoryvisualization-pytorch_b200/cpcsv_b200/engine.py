@@ -10,6 +10,7 @@ wgrad) are single-pass bf16; statistics, normalisation and all gradients are fp3
 import weakref
 
 import torch
+import torch.nn.functional as F
 
 from . import conv, ops
 from .ops import ACT_NONE, ACT_RELU, ACT_LRELU, BF16  # noqa: F401
@@ -189,6 +190,12 @@ def _e(shape, dev, dtype=torch.float32):
     return torch.empty(shape, device=dev, dtype=dtype)
 
 
+def _row_pad_map(rows, rows_pad, dev):
+    m = torch.full((rows_pad,), -1, dtype=torch.int32, device=dev)
+    m[:rows] = torch.arange(rows, dtype=torch.int32, device=dev)
+    return m
+
+
 class StateOrder:
     """In-place module state that several network calls update (BatchNorm running statistics,
     num_batches_tracked) must be updated in program order even when the calls run on different
@@ -284,11 +291,52 @@ class AuxBranch:
 
 # ------------------------------------------------------------------------------ conv nodes
 CONV_GEOM = {
-    # kind: (kernel, fwd pack kind, dgrad pack kind, wgrad taps, unpack kind, out scale)
+    # kind: (job kernel, fwd pack kind, dgrad pack kind, wgrad taps, unpack kind)
     "s1": (3, 0, 1, 9, 0),
     "up": (3, 2, 3, 16, 2),
     "s2": (4, 0, 1, 16, 0),
+    # 3x3 stride 2 pad 1 as the 4x4 "s2" job: the same input coordinate 2*o + k - 1, with the 4th row and
+    # column of the packed weight zero
+    "s2k3": (4, 0, 1, 16, 0),
 }
+# geometries whose weight kernel is smaller than the job's (zero-padded to it): kind -> weight kernel
+WEIGHT_KERNEL = {"s2k3": 3}
+
+
+def pack_taps(cache, w, w4, kindcode, rows_pad, cols_pad, planes, dtype):
+    """(cached) tap-major operand planes of ``w4()``, a 4-D ``[Co, Ci, kh, kw]`` view of parameter ``w``
+    (cpcsv_pack_conv_weight handles any kh x kw); a plain entry, re-packed when the parameter changed"""
+    def build():
+        ntap = w4().shape[2] * w4().shape[3]
+        t16 = ops.TORCH16[dtype]
+        hi = _e((ntap * rows_pad, cols_pad), w.device, t16)
+        lo = _e((ntap * rows_pad, cols_pad), w.device, t16) if planes == 2 else None
+        ops.pack_conv_weight(w4(), kindcode, rows_pad, cols_pad, hi, lo, dtype)
+        return [hi, lo]
+    return cache.get((id(w), "taps", kindcode, planes, dtype), w, build)
+
+
+def pack_im2col_weight(cache, w, kind, K_pad, planes=1, dtype=BF16):
+    """(cached) weight of an im2col'd convolution, columns k = tap * Ci + c (the order of cpcsv_im2col_small):
+    ``"fwd"``: the B operand of the forward GEMM, ``[hi, lo]`` planes ``[Co_pad, K_pad]``; ``"bwd"``: the B operand
+    of the data-gradient GEMM (into the im2col matrix), one bf16 plane ``[K_pad, Co_pad]``"""
+    Co = w.shape[0]
+    K, Cop = w.shape[1:].numel(), rup(Co, 64)
+    if kind == "bwd":
+        planes, dtype = 1, BF16
+
+    def build():
+        w2 = w.detach().reshape(Co, w.shape[1], -1).permute(0, 2, 1).reshape(Co, K).contiguous()
+        t16 = ops.TORCH16[dtype]
+        if kind == "fwd":
+            hi = _e((Cop, K_pad), w.device, t16)
+            lo = _e((Cop, K_pad), w.device, t16) if planes == 2 else None
+            ops.pack_matrix(w2, Cop, K_pad, K, K, 1, _row_pad_map(Co, Cop, w.device), hi, lo, dtype)
+        else:
+            hi, lo = _e((K_pad, Cop), w.device, t16), None
+            ops.pack_matrix(w2, K_pad, Cop, Co, 1, K, _row_pad_map(K, K_pad, w.device), hi, None)
+        return [hi, lo]
+    return cache.get((id(w), "im2col", kind, planes, dtype), w, build)
 
 
 def pack_conv(cache, w, geom, kindcode, rows_pad, cols_pad, planes, dtype=BF16):
@@ -337,8 +385,12 @@ def attach_stats(tape, job, out, wanted):
 
 
 class ConvNode:
-    """3x3 s1 / nearest-x2+3x3 / 4x4 s2 convolution, optionally spectrally normalised
-    (weight = weight_orig / sigma applied as the epilogue scalar alpha)."""
+    """3x3 s1 / nearest-x2+3x3 / 4x4 s2 / 3x3 s2 (``s2k3``) convolution, optionally spectrally normalised
+    (weight = weight_orig / sigma applied as the epilogue scalar alpha).
+
+    A 4-D weight whose kernel is the job's gets the persistent operand planes optim.PackedAdam keeps
+    current (pack_conv); any other weight -- a Conv3d ``[Co, Ci, 1, k, k]``, a 3x3 weight run as the 4x4 job
+    -- is packed from its 4-D (zero-padded) tap view into a plain cache entry (pack_taps)."""
 
     def __init__(self, tape, kind, x, weight, name, sn=None, alpha=None, bn_stats=False):
         self.tape, self.kind, self.x, self.w, self.name, self.sn = tape, kind, x, weight, name, sn
@@ -350,14 +402,24 @@ class ConvNode:
         N, H, W = x.N, x.H, x.W
         if kind == "up":
             H, W = 2 * H, 2 * W
-        elif kind == "s2":
+        elif kind != "s1":
             H, W = H // 2, W // 2
         self.out = T4(N, H, W, self.Co_pad)
         self.alpha = alpha          # 1/sigma of a spectral norm whose power iteration already ran
         self.dW = None
 
+    def _w4(self):
+        k = CONV_GEOM[self.kind][0]
+        wk = WEIGHT_KERNEL.get(self.kind, k)
+        w = self.w.detach()
+        w4 = w.view(w.shape[0], w.shape[1], wk, wk)
+        return w4 if wk == k else F.pad(w4, (0, k - wk, 0, k - wk)).contiguous()
+
     def _pack(self, kindcode, rows_pad, cols_pad, planes, dtype=BF16):
-        return pack_conv(self.tape.cache, self.w, self.kind, kindcode, rows_pad, cols_pad, planes, dtype)
+        w, k = self.w, CONV_GEOM[self.kind][0]
+        if w.dim() == 4 and w.shape[2] == w.shape[3] == k:
+            return pack_conv(self.tape.cache, w, self.kind, kindcode, rows_pad, cols_pad, planes, dtype)
+        return pack_taps(self.tape.cache, w, self._w4, kindcode, rows_pad, cols_pad, planes, dtype)
 
     def forward(self):
         t, x, out = self.tape, self.x, self.out
@@ -368,11 +430,11 @@ class ConvNode:
         out.f32 = _e((out.N, out.H, out.W, out.C), dev)
         xp = x.planes(t.planes)
         if self.kind == "s1":
-            job = conv.conv_s1_fwd(xp, wp, out.f32, 3, self.alpha, dtype=t.dtype)
+            job = conv.conv_s1_fwd(xp, wp, out.f32, 3, self.alpha, dtype=t.dtype, splits=t.splits)
         elif self.kind == "up":
             job = conv.upconv_fwd(xp, wp, out.f32, dtype=t.dtype)
         else:
-            job = conv.conv_s2_fwd(xp, wp, out.f32, self.alpha, dtype=t.dtype)
+            job = conv.conv_s2_fwd(xp, wp, out.f32, self.alpha, dtype=t.dtype, splits=t.splits)
         attach_stats(t, job, out, self.bn_stats)
         ops.conv_gemm(job)
 
@@ -381,7 +443,7 @@ class ConvNode:
         dz = out.grad16
         assert dz is not None, self.name
         dev = dz.device
-        k, _, dkind, ntap, ukind = CONV_GEOM[self.kind]
+        dkind = CONV_GEOM[self.kind][2]
         if x.needs_grad:
             # data gradient first: it is what the rest of the backward chain waits for
             wt = self._pack(dkind, self.Ci_pad, self.Co_pad, 1)[0]
@@ -403,7 +465,8 @@ class ConvNode:
     def _wgrad(self, dz):
         x = self.x
         dev = dz.device
-        _k, _f, _d, ntap, ukind = CONV_GEOM[self.kind]
+        k, _f, _d, ntap, ukind = CONV_GEOM[self.kind]
+        wk = WEIGHT_KERNEL.get(self.kind, k)
         dwt = _e((ntap, self.Co_pad, self.Ci_pad), dev)
         if self.kind == "s1":
             job = conv.conv_s1_wgrad(dz, x.hi, dwt, 3)
@@ -412,16 +475,144 @@ class ConvNode:
         else:
             job = conv.conv_s2_wgrad(dz, x.hi, dwt)
         ops.conv_gemm(job)
-        g = _e(tuple(self.w.shape), dev)
-        if self.sn is not None and ukind in (0, 2):
+        if self.sn is not None and wk == k:
             # spectral norm: sum(dW_eff .* W_orig) comes out of the same pass that un-packs the gradient
+            g = _e(tuple(self.w.shape), dev)
             dot = torch.zeros(1, device=dev)
             ops.unpack_conv_wgrad_dot(dwt, self.Co_pad * self.Ci_pad, self.Ci_pad, ukind, None, g,
                                       self.w.detach(), dot)
             self.dW = self.sn.backward(g, self.w, dot)
+            return
+        g = _e((self.Co, self.Ci, k, k) if wk != k else tuple(self.w.shape), dev)
+        ops.unpack_conv_wgrad(dwt, self.Co_pad * self.Ci_pad, self.Ci_pad, ukind, None, g)
+        if wk != k:     # zero-padded kernel: keep the taps the weight has
+            g = g[:, :, :wk, :wk].contiguous().view(self.w.shape)
+        self.dW = self.sn.backward(g, self.w) if self.sn is not None else g
+
+
+class TemporalNode:
+    """Conv3d (3, 1, 1) stride (s, 1, 1) pad (1, 0, 0), s = 1 or 2, optionally spectrally normalised (alpha =
+    1/sigma): [B, T, HW, Ci] -> [B, To, HW, Co] on ``[B * T, H, W, C]`` activations.  Backward: stride 2 only."""
+
+    def __init__(self, tape, x, B, weight, name, stride, sn=None, alpha=None):
+        self.tape, self.x, self.B, self.w, self.name, self.stride = tape, x, B, weight, name, stride
+        self.sn, self.alpha = sn, alpha
+        self.Co, self.Ci = weight.shape[0], weight.shape[1]
+        self.Co_pad, self.Ci_pad = rup(self.Co, 64), x.C
+        assert rup(self.Ci, 64) == x.C and x.N % B == 0 and stride in (1, 2), name
+        self.T = x.N // B
+        self.To = self.T if stride == 1 else (self.T - 1) // 2 + 1
+        self.out = T4(B * self.To, x.H, x.W, self.Co_pad)
+        self.dW = None
+
+    def _w4(self):
+        w = self.w.detach()
+        return w.view(w.shape[0], w.shape[1], 3, 1)
+
+    def _pack(self, kindcode, rows_pad, cols_pad, planes, dtype=BF16):
+        return pack_taps(self.tape.cache, self.w, self._w4, kindcode, rows_pad, cols_pad, planes, dtype)
+
+    def _v(self, t, frames):
+        return t.view(self.B, frames, self.x.H * self.x.W, t.shape[-1]) if t is not None else None
+
+    def forward(self):
+        t, x, out = self.tape, self.x, self.out
+        wp = self._pack(0, self.Co_pad, self.Ci_pad, t.planes, t.dtype)
+        out.f32 = _e((out.N, out.H, out.W, out.C), x.hi.device)
+        xp = [self._v(p, self.T) for p in x.planes(t.planes)]
+        if self.stride == 1:
+            jobs = [conv.conv_t3s1_fwd(xp, wp, self._v(out.f32, self.To), self.alpha, dtype=t.dtype,
+                                       splits=t.splits)]
         else:
-            ops.unpack_conv_wgrad(dwt, self.Co_pad * self.Ci_pad, self.Ci_pad, ukind, None, g)
-            self.dW = self.sn.backward(g, self.w) if self.sn is not None else g
+            jobs = conv.conv_t3_fwd(xp, wp, self._v(out.f32, self.To), self.alpha, dtype=t.dtype)
+        for job in jobs:
+            ops.conv_gemm(job)
+
+    def backward(self, need_wgrad=True):
+        x, out = self.x, self.out
+        dz = out.grad16
+        assert dz is not None and self.stride == 2, self.name
+        dz5 = self._v(dz, self.To)
+        if x.needs_grad:
+            assert x.grad is None
+            wt = self._pack(1, self.Ci_pad, self.Co_pad, 1)[0]
+            x.grad = _e((x.N, x.H, x.W, x.C), dz.device)
+            for job in conv.conv_t3_dgrad(dz5, wt, self._v(x.grad, self.T), self.alpha):
+                ops.conv_gemm(job)
+        if need_wgrad:
+            self.tape.aux.run(lambda: self._wgrad(dz5), dz)
+        out.grad16 = None
+
+    def _wgrad(self, dz5):
+        dev = dz5.device
+        # zeroed: the even- and odd-frame jobs accumulate into it (and for T == 1 taps 0 / 2 have no job at all)
+        dwt = torch.zeros((3, self.Co_pad, self.Ci_pad), device=dev)
+        for job in conv.conv_t3_wgrad(dz5, self._v(self.x.hi, self.T), dwt):
+            ops.conv_gemm(job)
+        g = _e((self.Co, self.Ci, 3, 1), dev)
+        ops.unpack_conv_wgrad(dwt, self.Co_pad * self.Ci_pad, self.Ci_pad, 0, None, g)
+        g = g.view(self.w.shape)
+        self.dW = self.sn.backward(g, self.w) if self.sn is not None else g
+
+
+class Im2colNode:
+    """k x k convolution (stride, pad, no bias) of a few-channel NCHW fp32 image ``img`` as im2col + one GEMM,
+    K = k*k*Ci padded to a multiple of 64, optionally spectrally normalised (alpha = 1/sigma, the epilogue
+    scalar).  Output: T4 with the fp32 conv output; ``backward`` returns d(img) [n, Ci, H, W] fp32."""
+
+    def __init__(self, tape, img, weight, name, stride, pad, sn=None, alpha=None):
+        self.tape, self.img, self.w, self.name, self.stride, self.pad = tape, img, weight, name, stride, pad
+        self.sn, self.alpha = sn, alpha
+        n, Ci, H, W = img.shape
+        self.Co, self.k = weight.shape[0], weight.shape[-1]
+        assert weight.shape[1] == Ci, name
+        self.K_pad = rup(self.k * self.k * Ci, 64)
+        Ho, Wo = (H + 2 * pad - self.k) // stride + 1, (W + 2 * pad - self.k) // stride + 1
+        self.out = T4(n, Ho, Wo, rup(self.Co, 64))
+        self.col = self.dW = None
+
+    def forward(self):
+        t, out, Kp = self.tape, self.out, self.K_pad
+        dev = self.img.device
+        t16 = ops.TORCH16[t.dtype]
+        col = T4(out.N, out.H, out.W, Kp)
+        col.hi = _e((out.N, out.H, out.W, Kp), dev, t16)
+        col.lo = _e((out.N, out.H, out.W, Kp), dev, t16) if t.planes == 2 else None
+        ops.im2col_small(self.img.detach(), self.k, self.stride, self.pad, col.hi, col.lo, Kp, t.dtype)
+        if self.sn is not None and self.alpha is None:
+            self.alpha = self.sn.forward(self.w, t.training, t.need_grad)
+        out.f32 = _e((out.N, out.H, out.W, out.C), dev)
+        ops.conv_gemm(conv.gemm_nt([col.hi.view(-1, Kp), col.lo.view(-1, Kp) if col.lo is not None else None],
+                                   pack_im2col_weight(t.cache, self.w, "fwd", Kp, t.planes, t.dtype),
+                                   out.f32.view(-1, out.C), alpha=self.alpha, dtype=t.dtype, splits=t.splits))
+        col.lo = None
+        if t.need_grad:
+            self.col = col      # the weight gradient multiplies with it
+
+    def backward(self, need_wgrad=True, need_dx=True):
+        """consumes out.grad16"""
+        dz = self.out.grad16.view(-1, self.out.C)
+        dev = dz.device
+        Kp = self.K_pad
+        if need_wgrad:
+            def wgrad():
+                d = _e((self.out.C, Kp), dev)
+                ops.conv_gemm(conv.gemm_tn(dz, self.col.hi.view(-1, Kp), d))
+                Ci = self.w.shape[1]
+                g = d[:self.Co, :self.k * self.k * Ci].reshape(self.Co, -1, Ci).permute(0, 2, 1).contiguous()
+                g = g.view(self.w.shape)
+                self.dW = self.sn.backward(g, self.w) if self.sn is not None else g
+            self.tape.aux.run(wgrad, dz)
+        dx = None
+        if need_dx:
+            n, Ci, H, W = self.img.shape
+            dcol = _e((dz.shape[0], Kp), dev)
+            ops.conv_gemm(conv.gemm_nt([dz, None], pack_im2col_weight(self.tape.cache, self.w, "bwd", Kp), dcol,
+                                       alpha=self.alpha))
+            dx = _e((n, Ci, H, W), dev)
+            ops.col2im_small(dcol, n, Ci, H, W, self.k, self.stride, self.pad, dx)
+        self.out.grad16 = None
+        return dx
 
 
 class SpectralNorm:
@@ -480,7 +671,8 @@ class GemmNode:
         dev = x.hi.device
         out.f32 = _e((out.N, out.H, out.W, out.C), dev)
         a = [p.view(x.rows, x.C) if p is not None else None for p in x.planes(t.planes)]
-        job = conv.gemm_nt(a, self.pack_fwd(t.planes, t.dtype), out.f32.view(x.rows, self.npad), dtype=t.dtype)
+        job = conv.gemm_nt(a, self.pack_fwd(t.planes, t.dtype), out.f32.view(x.rows, self.npad), dtype=t.dtype,
+                           splits=t.splits)
         attach_stats(t, job, out, self.bn_stats)
         ops.conv_gemm(job)
 
@@ -616,12 +808,18 @@ class Tape:
     """One network call.  With ``need_grad`` the forward GEMMs use bf16 hi/lo split operands
     (3 MMAs); a no-grad call (the fakes for the discriminator update, inference) uses single-pass
     fp16 operands -- SURVEY.md Appendix E: fp16, not bf16, keeps the discriminator gradients that
-    are computed on those fakes within tolerance."""
+    are computed on those fakes within tolerance.
+
+    ``split_k=False``: no forward GEMM splits its reduction (the nearest-x2 "up" convolution of the generator
+    always picks its own split).  Split-K partial sums meet in fp32 atomics in
+    whatever order they arrive; without them every output is bit-for-bit reproducible."""
 
     STAT_CHUNK = 1 << 15       # fp64 slots per zero-filled arena chunk (override per network call)
 
-    def __init__(self, cache, training=True, need_grad=True, planes=None, dtype=None, stat_chunk=None):
+    def __init__(self, cache, training=True, need_grad=True, planes=None, dtype=None, stat_chunk=None,
+                 split_k=True):
         self.cache, self.training, self.need_grad = cache, training, need_grad
+        self.splits = None if split_k else 1    # the forward job builders' `splits` (None: conv.pick_splits)
         self._arena, self._arena_used = None, 0
         self._chunk = stat_chunk if stat_chunk is not None else self.STAT_CHUNK
         split = need_grad or NOGRAD_SPLIT

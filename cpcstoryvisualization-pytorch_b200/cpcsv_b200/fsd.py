@@ -7,29 +7,31 @@ features in front of ``fc``) in eval mode, on stories preprocessed as documented
 Every Conv3d of that network is (1, k, k) or (k, 1, 1); on channels-last activations ``[B * T, H, W, C]``
 (frames as batch entries) each is an implicit GEMM the tcgen05 kernel runs with bf16 hi/lo split operands:
 
-* stem (1, 7, 7) stride (1, 2, 2) pad (0, 3, 3) on 3 channels: im2col (K = 147 -> 192) + one GEMM, as the
-  stem of the order-consistency critic (video.py);
-* (3, 1, 1) stride 1 pad (1, 0, 0): ``conv.conv_t3s1_fwd`` on ``[B, T, HW, C]`` (one job, three frame taps);
-* (3, 1, 1) stride (2, 1, 1) pad (1, 0, 0): ``conv.conv_t3_fwd`` (even / odd frames);
-* (1, 3, 3) stride 1 pad (0, 1, 1): ``conv.conv_s1_fwd`` with frames as batch entries;
-* (1, 3, 3) stride (1, 2, 2) pad (0, 1, 1): the 4x4 / stride-2 parity job with a zero 4th row / column;
+* stem (1, 7, 7) stride (1, 2, 2) pad (0, 3, 3) on 3 channels: im2col (K = 147 -> 192) + one GEMM
+  (engine.Im2colNode, as the stem of the order-consistency critic);
+* (3, 1, 1) stride 1 pad (1, 0, 0): engine.TemporalNode, ``conv.conv_t3s1_fwd`` on ``[B, T, HW, C]`` (one job,
+  three frame taps);
+* (3, 1, 1) stride (2, 1, 1) pad (1, 0, 0): engine.TemporalNode, ``conv.conv_t3_fwd`` (even / odd frames);
+* (1, 3, 3) stride 1 pad (0, 1, 1): engine.ConvNode ``s1`` with frames as batch entries;
+* (1, 3, 3) stride (1, 2, 2) pad (0, 1, 1): engine.ConvNode ``s2k3``, the 4x4 / stride-2 parity job with a zero
+  4th row / column;
 * (1, 1, 1) stride (2, 2, 2) shortcut projection: ``conv.conv_p2_fwd`` (one job per output frame).
 
 Inner BatchNorm + ReLU: engine.BnActNode with the running statistics.  The end of a residual block (its last
 BatchNorm, the shortcut's BatchNorm, the add, the ReLU) is one ``cpcsv_bn_add_act_pack`` launch.  Channel
 counts are padded to multiples of 64 (stem 45, mid-planes 144 / 230 / 288 / 460 / 576 / 921 / 1152).
-Forward only, eval mode only, under ``torch.no_grad()``.  No job splits its reduction (split-K partial sums
-meet in fp32 atomics, in whatever order they arrive): a story's features are bit-for-bit reproducible and do not
-depend on the other stories of its chunk, so the FSD of the same stories is the same number every time.
+Forward only, eval mode only, under ``torch.no_grad()``.  The tape runs with ``split_k=False``, so no job splits
+its reduction (split-K partial sums meet in fp32 atomics, in whatever order they arrive): a story's features
+are bit-for-bit reproducible and do not depend on the other stories of its chunk, so the FSD of the same
+stories is the same number every time.
 """
 import numpy as np
 import torch
 import torch.nn as nn
 
 from . import conv, ops
-from .engine import T4, BnActNode, Tape, eval_affine, rup, _e
-from .nets import _CACHE, _bn_tuple, _row_pad_map
-from .video import STEM_K, _pack_generic
+from .engine import T4, BnActNode, ConvNode, Im2colNode, Tape, TemporalNode, eval_affine, pack_taps, rup, _e
+from .nets import _CACHE, _bn_tuple
 
 # torchvision's Kinetics-400 normalisation of the R(2+1)D-18 weights (the reference feeds 64 x 64 frames to
 # the network without a resize, SURVEY.md Appendix D)
@@ -136,64 +138,6 @@ def _drop_fc(module, state_dict, prefix, *args):
 
 
 # ------------------------------------------------------------------------------------------ tape nodes
-class FrameConvNode:
-    """Conv3d (1, 3, 3) stride (1, s, s) pad (0, 1, 1), frames as batch entries: [N, H, W, Ci] -> [N, H/s, W/s, Co].
-    Stride 2 runs as the 4x4 / stride-2 parity job with a zero 4th row and column (video.SpatialNode)."""
-
-    def __init__(self, tape, x, weight, stride, name):
-        self.tape, self.x, self.w, self.stride, self.name = tape, x, weight, stride, name
-        self.Co, self.Co_pad, self.Ci_pad = weight.shape[0], rup(weight.shape[0], 64), x.C
-        assert rup(weight.shape[1], 64) == x.C and stride in (1, 2), name
-        self.out = T4(x.N, x.H // stride, x.W // stride, self.Co_pad)
-
-    def _w4(self):
-        w = self.w.detach()
-        w3 = w.view(w.shape[0], w.shape[1], 3, 3)
-        return w3 if self.stride == 1 else nn.functional.pad(w3, (0, 1, 0, 1)).contiguous()
-
-    def forward(self):
-        t, x, out = self.tape, self.x, self.out
-        tag = "r133" if self.stride == 1 else "r133s2"
-        wp = _pack_generic(t.cache, self.w, self._w4, tag, 0, self.Co_pad, self.Ci_pad, t.planes, t.dtype)
-        out.f32 = _e((out.N, out.H, out.W, out.C), x.hi.device)
-        xp = x.planes(t.planes)
-        if self.stride == 1:
-            ops.conv_gemm(conv.conv_s1_fwd(xp, wp, out.f32, 3, dtype=t.dtype, splits=1))
-        else:
-            ops.conv_gemm(conv.conv_s2_fwd(xp, wp, out.f32, dtype=t.dtype, splits=1))
-
-
-class TemporalConvNode:
-    """Conv3d (3, 1, 1) stride (s, 1, 1) pad (1, 0, 0): [B, T, HW, Ci] -> [B, To, HW, Co]"""
-
-    def __init__(self, tape, x, B, weight, stride, name):
-        self.tape, self.x, self.B, self.w, self.stride, self.name = tape, x, B, weight, stride, name
-        self.Co_pad, self.Ci_pad = rup(weight.shape[0], 64), x.C
-        assert rup(weight.shape[1], 64) == x.C and x.N % B == 0 and stride in (1, 2), name
-        self.T = x.N // B
-        self.To = self.T if stride == 1 else (self.T - 1) // 2 + 1
-        self.out = T4(B * self.To, x.H, x.W, self.Co_pad)
-
-    def _w4(self):
-        w = self.w.detach()
-        return w.view(w.shape[0], w.shape[1], 3, 1)
-
-    def _v(self, t, frames):
-        return t.view(self.B, frames, self.x.H * self.x.W, t.shape[-1]) if t is not None else None
-
-    def forward(self):
-        t, x, out = self.tape, self.x, self.out
-        wp = _pack_generic(t.cache, self.w, self._w4, "r311", 0, self.Co_pad, self.Ci_pad, t.planes, t.dtype)
-        out.f32 = _e((out.N, out.H, out.W, out.C), x.hi.device)
-        xp = [self._v(p, self.T) for p in x.planes(t.planes)]
-        if self.stride == 1:
-            jobs = [conv.conv_t3s1_fwd(xp, wp, self._v(out.f32, self.To), dtype=t.dtype, splits=1)]
-        else:
-            jobs = conv.conv_t3_fwd(xp, wp, self._v(out.f32, self.To), dtype=t.dtype)
-        for job in jobs:
-            ops.conv_gemm(job)
-
-
 class ShortcutNode:
     """Conv3d (1, 1, 1) stride (2, 2, 2), the projected shortcut: [B, T, H, W, Ci] -> [B, To, H/2, W/2, Co]"""
 
@@ -211,11 +155,11 @@ class ShortcutNode:
 
     def forward(self):
         t, x, out = self.tape, self.x, self.out
-        wp = _pack_generic(t.cache, self.w, self._w4, "r111s2", 0, self.Co_pad, self.Ci_pad, t.planes, t.dtype)
+        wp = pack_taps(t.cache, self.w, self._w4, 0, self.Co_pad, self.Ci_pad, t.planes, t.dtype)
         out.f32 = _e((out.N, out.H, out.W, out.C), x.hi.device)
         xp = [p.view(self.B, self.T, x.H, x.W, x.C) for p in x.planes(t.planes) if p is not None]
         for job in conv.conv_p2_fwd(xp, wp, out.f32.view(self.B, self.To, out.H, out.W, out.C), dtype=t.dtype,
-                                    splits=1):
+                                    splits=t.splits):
             ops.conv_gemm(job)
 
 
@@ -252,41 +196,15 @@ class FeatureRunner:
     def __init__(self, net):
         self.net = net
 
-    def _pack_stem(self, planes, dtype):
-        w = self.net.stem[0].weight
-        Co, K = w.shape[0], w.shape[1] * 49
-        Cop = rup(Co, 64)
-
-        def build():
-            w2 = w.detach().view(Co, w.shape[1], 7, 7).permute(0, 2, 3, 1).reshape(Co, K).contiguous()
-            t16 = ops.TORCH16[dtype]
-            hi = _e((Cop, STEM_K), w.device, t16)
-            lo = _e((Cop, STEM_K), w.device, t16) if planes == 2 else None
-            ops.pack_matrix(w2, Cop, STEM_K, K, K, 1, _row_pad_map(Co, Cop, w.device), hi, lo, dtype)
-            return [hi, lo]
-        return _CACHE.get((id(w), "r177", planes, dtype), w, build)
-
     def run(self, frames, T):
         """frames: normalised fp32 [B * T, 3, H, W] (n = b * T + t) -> fp32 [B, 512]"""
         net = self.net
         stem = net.stem
-        dev = frames.device
-        N, Cin, H, W = frames.shape
-        B = N // T
-        tape = Tape(_CACHE, training=False, need_grad=False, planes=2, dtype=ops.BF16)
-        t16 = ops.TORCH16[tape.dtype]
-        Ho, Wo = H // 2, W // 2
-        col_hi = _e((N, Ho, Wo, STEM_K), dev, t16)
-        col_lo = _e((N, Ho, Wo, STEM_K), dev, t16)
-        ops.im2col_small(frames, 7, 2, 3, col_hi, col_lo, STEM_K, tape.dtype)
-        z0 = T4(N, Ho, Wo, rup(stem[0].weight.shape[0], 64))
-        z0.f32 = _e((N, Ho, Wo, z0.C), dev)
-        ops.conv_gemm(conv.gemm_nt([col_hi.view(-1, STEM_K), col_lo.view(-1, STEM_K)],
-                                   self._pack_stem(tape.planes, tape.dtype), z0.f32.view(-1, z0.C), dtype=tape.dtype,
-                                   splits=1))
-        del col_hi, col_lo
+        B = frames.shape[0] // T
+        tape = Tape(_CACHE, training=False, need_grad=False, planes=2, dtype=ops.BF16, split_k=False)
+        z0 = tape.add(Im2colNode(tape, frames, stem[0].weight, "fsd.stem.0", 2, 3))
         a = tape.add(BnActNode(tape, z0, _bn_tuple(stem[1]), ops.ACT_RELU, "fsd.stem.1"))
-        z = tape.add(TemporalConvNode(tape, a, B, stem[3].weight, 1, "fsd.stem.3"))
+        z = tape.add(TemporalNode(tape, a, B, stem[3].weight, "fsd.stem.3", 1))
         # fp32 values too: the identity shortcut of layer1.0
         a = tape.add(BnActNode(tape, z, _bn_tuple(stem[4]), ops.ACT_RELU, "fsd.stem.4", want_f32=True))
         blocks = net.blocks()
@@ -300,13 +218,13 @@ class FeatureRunner:
     def _block(tape, x, B, blk, name, last):
         c1, c2 = blk.conv1[0], blk.conv2[0]
         s = blk.stride
-        m = tape.add(FrameConvNode(tape, x, c1[0].weight, s, name + ".conv1.0.0"))
+        m = tape.add(ConvNode(tape, "s1" if s == 1 else "s2k3", x, c1[0].weight, name + ".conv1.0.0"))
         m = tape.add(BnActNode(tape, m, _bn_tuple(c1[1]), ops.ACT_RELU, name + ".conv1.0.1"))
-        z = tape.add(TemporalConvNode(tape, m, B, c1[3].weight, s, name + ".conv1.0.3"))
+        z = tape.add(TemporalNode(tape, m, B, c1[3].weight, name + ".conv1.0.3", s))
         a = tape.add(BnActNode(tape, z, _bn_tuple(blk.conv1[1]), ops.ACT_RELU, name + ".conv1.1"))
-        m = tape.add(FrameConvNode(tape, a, c2[0].weight, 1, name + ".conv2.0.0"))
+        m = tape.add(ConvNode(tape, "s1", a, c2[0].weight, name + ".conv2.0.0"))
         m = tape.add(BnActNode(tape, m, _bn_tuple(c2[1]), ops.ACT_RELU, name + ".conv2.0.1"))
-        z = tape.add(TemporalConvNode(tape, m, B, c2[3].weight, 1, name + ".conv2.0.3"))
+        z = tape.add(TemporalNode(tape, m, B, c2[3].weight, name + ".conv2.0.3", 1))
         r, rbn = x, None
         if blk.downsample is not None:
             r = tape.add(ShortcutNode(tape, x, B, blk.downsample[0].weight, name + ".downsample.0"))

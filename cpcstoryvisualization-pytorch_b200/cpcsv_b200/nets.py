@@ -8,7 +8,7 @@ Reference call sites: generator trunk ``model.py:379-407 / 445-470``; encoders
 import torch
 
 from . import conv, engine, ops
-from .engine import T4, BnActNode, ConvNode, GemmNode, SpectralNorm, Tape, rup, _e
+from .engine import T4, BnActNode, ConvNode, GemmNode, SpectralNorm, Tape, pack_im2col_weight, rup, _e, _row_pad_map
 
 _CACHE = engine.WeightCache()
 
@@ -526,12 +526,6 @@ def _pad4(x):
     return out
 
 
-def _row_pad_map(rows, rows_pad, dev):
-    m = torch.full((rows_pad,), -1, dtype=torch.int32, device=dev)
-    m[:rows] = torch.arange(rows, dtype=torch.int32, device=dev)
-    return m
-
-
 # =============================================================================== D encoder
 class EncoderRunner:
     """encode_img: conv4x4 s2 -> LeakyReLU (one direct kernel, csrc/enc0.cu), then 3 x
@@ -555,21 +549,6 @@ class EncoderRunner:
     def _w0(self):
         enc0 = self.D.encode_img[0]
         return enc0.weight_orig if self.sn0 else enc0.weight
-
-    def _pack0(self):
-        """layer-0 weight as the B operand of the data-gradient GEMM: [64, Co_pad] with row tap*Ci + c"""
-        w = self._w0()
-        Co, Ci = w.shape[0], w.shape[1]
-        Cop = rup(Co, 64)
-        K = 16 * Ci
-        assert K <= 64
-
-        def build():
-            w2 = w.detach().permute(0, 2, 3, 1).reshape(Co, K).contiguous()     # [co, tap*Ci + c]
-            hi = _e((64, Cop), w.device, torch.bfloat16)                         # [k, co]
-            ops.pack_matrix(w2, 64, Cop, Co, 1, K, _row_pad_map(K, 64, w.device), hi, None)
-            return hi
-        return _CACHE.get((id(w), "enc0_bwd", 2), w, build)
 
     def run_forward(self, x, *plist):
         D = self.D
@@ -668,7 +647,9 @@ class EncoderRunner:
         if needs[0]:
             n, Cin, H, W = self.x_shape
             dcol = _e((dz0m.shape[0], 64), dev)
-            ops.conv_gemm(conv.gemm_nt([dz0m, None], [self._pack0(), None], dcol, alpha=self.alpha0))
+            # layer-0 weight as the B operand: [64, Co_pad] with row tap*Ci + c
+            ops.conv_gemm(conv.gemm_nt([dz0m, None], pack_im2col_weight(_CACHE, w0, "bwd", 64), dcol,
+                                       alpha=self.alpha0))
             dx = _e((n, Cin, H, W), dev)
             ops.col2im_small(dcol, n, Cin, H, W, 4, 2, 1, dx)
         out = [dx]

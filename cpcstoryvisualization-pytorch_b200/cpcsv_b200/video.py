@@ -4,14 +4,16 @@
 Every Conv3d of the reference is (1, k, k) or (k, 1, 1), so on channels-last activations
 ``[B * T, H, W, C]`` each one is an implicit GEMM the tcgen05 kernel already runs:
 
-* stem conv (1, 7, 7) stride (1, 2, 2), 3 input channels: im2col (K = 147 -> 192) + one GEMM, like the first
-  layer of the image discriminators;
+* stem conv (1, 7, 7) stride (1, 2, 2), 3 input channels: im2col (K = 147 -> 192) + one GEMM
+  (engine.Im2colNode);
 * stem conv (1, 1, 1) with TEMPORAL padding 1 (model.py:109-111; T -> T + 2, the two new frames are zero
   before the BatchNorm and relu(beta) after it): a 1-tap GEMM written into frames 1..T of a zero-filled
   ``[B, T + 2, HW, C]`` tensor through the job's output strides;
-* (1, 3, 3) stride (1, 2, 2) pad (0, 1, 1): the 4x4 / stride-2 parity-view job with a zero 4th row / column
-  (the cascade generator's downBlock geometry), frames folded into the batch dimension;
-* (3, 1, 1) stride (2, 1, 1) pad (1, 0, 0): conv.conv_t3_* on ``[B, T, HW, C]`` views (even / odd frames).
+* (1, 3, 3) stride (1, 2, 2) pad (0, 1, 1): engine.ConvNode's ``s2k3`` geometry, the 4x4 / stride-2 parity-view
+  job with a zero 4th row / column (the cascade generator's downBlock geometry), frames folded into the batch
+  dimension;
+* (3, 1, 1) stride (2, 1, 1) pad (1, 0, 0): engine.TemporalNode, conv.conv_t3_* on ``[B, T, HW, C]`` views
+  (even / odd frames).
 
 All convs are spectrally normalised (1 / sigma is the GEMM's epilogue scalar), followed by a batch-statistics
 BatchNorm3d (= per-channel statistics over all B*T*H*W rows) and ReLU / LeakyReLU(0.2): engine.BnActNode.
@@ -19,109 +21,14 @@ AdaptiveAvgPool3d(1) and the 4-layer detector (two spectral-norm Linears around 
 hundred floats per story: fp32 kernels of cpcsv_b200.functions.
 """
 import torch
-import torch.nn.functional as F
 
 from . import conv, ops
-from .engine import T4, BnActNode, ConvNode, SpectralNorm, Tape, rup, _e
-from .nets import _CACHE, TapeFn, _bn_tuple, _eval_bn_unsupported, _row_pad_map
+from .engine import T4, BnActNode, ConvNode, Im2colNode, SpectralNorm, Tape, TemporalNode, pack_taps, rup, _e
+from .nets import _CACHE, TapeFn, _bn_tuple, _eval_bn_unsupported
 
 # (index inside story_encoder, geometry) after the stem; model.py:155-189
 LAYERS = ((1, "spatial"), (4, "temporal"), (7, "spatial"), (10, "temporal"), (13, "spatial"), (16, "temporal"),
           (19, "spatial"), (22, "temporal"))
-STEM_K = 192        # 7 * 7 * 3 = 147 im2col columns, padded to a multiple of 64
-
-
-def _pack_generic(cache, w, w4, tag, kindcode, rows_pad, cols_pad, planes, dtype):
-    """tap-major operand planes of the 4-D view ``w4`` of parameter ``w`` (cpcsv_pack_conv_weight handles any
-    kh x kw); cached per parameter version like every other re-layout"""
-    def build():
-        ntap = w4().shape[2] * w4().shape[3]
-        t16 = ops.TORCH16[dtype]
-        hi = _e((ntap * rows_pad, cols_pad), w.device, t16)
-        lo = _e((ntap * rows_pad, cols_pad), w.device, t16) if planes == 2 else None
-        ops.pack_conv_weight(w4(), kindcode, rows_pad, cols_pad, hi, lo, dtype)
-        return [hi, lo]
-    return cache.get((id(w), tag, kindcode, planes, dtype), w, build)
-
-
-class SpatialNode(ConvNode):
-    """Conv3d (1, 3, 3) stride (1, 2, 2) pad (0, 1, 1), spectral norm, frames as batch entries"""
-
-    def __init__(self, tape, x, weight, name, sn, alpha):
-        super().__init__(tape, "s2", x, weight, name, sn=sn, alpha=alpha, bn_stats=True)
-
-    def _w4(self):
-        w = self.w.detach()
-        return F.pad(w.view(w.shape[0], w.shape[1], 3, 3), (0, 1, 0, 1)).contiguous()
-
-    def _pack(self, kindcode, rows_pad, cols_pad, planes, dtype=ops.BF16):
-        return _pack_generic(self.tape.cache, self.w, self._w4, "v133", kindcode, rows_pad, cols_pad, planes, dtype)
-
-    def _wgrad(self, dz):
-        x, dev = self.x, dz.device
-        dwt = _e((16, self.Co_pad, self.Ci_pad), dev)
-        ops.conv_gemm(conv.conv_s2_wgrad(dz, x.hi, dwt))
-        g4 = _e((self.Co, self.Ci, 4, 4), dev)
-        ops.unpack_conv_wgrad(dwt, self.Co_pad * self.Ci_pad, self.Ci_pad, 0, None, g4)
-        g = g4[:, :, :3, :3].contiguous().view(self.w.shape)
-        self.dW = self.sn.backward(g, self.w)
-
-
-class TemporalNode:
-    """Conv3d (3, 1, 1) stride (2, 1, 1) pad (1, 0, 0), spectral norm: [B, T, HW, C] -> [B, (T - 1) // 2 + 1, HW, Co]"""
-
-    def __init__(self, tape, x, B, weight, name, sn, alpha):
-        self.tape, self.x, self.B, self.w, self.name, self.sn, self.alpha = tape, x, B, weight, name, sn, alpha
-        self.Co, self.Ci = weight.shape[0], weight.shape[1]
-        self.Co_pad, self.Ci_pad = rup(self.Co, 64), x.C
-        assert rup(self.Ci, 64) == x.C and x.N % B == 0
-        self.T = x.N // B
-        self.To = (self.T - 1) // 2 + 1
-        self.out = T4(B * self.To, x.H, x.W, self.Co_pad)
-        self.dW = None
-
-    def _w4(self):
-        w = self.w.detach()
-        return w.view(w.shape[0], w.shape[1], 3, 1)
-
-    def _pack(self, kindcode, rows_pad, cols_pad, planes, dtype=ops.BF16):
-        return _pack_generic(self.tape.cache, self.w, self._w4, "v311", kindcode, rows_pad, cols_pad, planes, dtype)
-
-    def _v(self, t, frames):
-        return t.view(self.B, frames, self.x.H * self.x.W, t.shape[-1]) if t is not None else None
-
-    def forward(self):
-        t, x, out = self.tape, self.x, self.out
-        wp = self._pack(0, self.Co_pad, self.Ci_pad, t.planes, t.dtype)
-        out.f32 = _e((out.N, out.H, out.W, out.C), x.hi.device)
-        for job in conv.conv_t3_fwd([self._v(p, self.T) for p in x.planes(t.planes)], wp,
-                                    self._v(out.f32, self.To), self.alpha, dtype=t.dtype):
-            ops.conv_gemm(job)
-
-    def backward(self, need_wgrad=True):
-        x, out = self.x, self.out
-        dz = out.grad16
-        assert dz is not None, self.name
-        dz5 = self._v(dz, self.To)
-        if x.needs_grad:
-            assert x.grad is None
-            wt = self._pack(1, self.Ci_pad, self.Co_pad, 1)[0]
-            x.grad = _e((x.N, x.H, x.W, x.C), dz.device)
-            for job in conv.conv_t3_dgrad(dz5, wt, self._v(x.grad, self.T), self.alpha):
-                ops.conv_gemm(job)
-        if need_wgrad:
-            self.tape.aux.run(lambda: self._wgrad(dz5), dz)
-        out.grad16 = None
-
-    def _wgrad(self, dz5):
-        dev = dz5.device
-        # zeroed: the even- and odd-frame jobs accumulate into it (and for T == 1 taps 0 / 2 have no job at all)
-        dwt = torch.zeros((3, self.Co_pad, self.Ci_pad), device=dev)
-        for job in conv.conv_t3_wgrad(dz5, self._v(self.x.hi, self.T), dwt):
-            ops.conv_gemm(job)
-        g = _e((self.Co, self.Ci, 3, 1), dev)
-        ops.unpack_conv_wgrad(dwt, self.Co_pad * self.Ci_pad, self.Ci_pad, 0, None, g)
-        self.dW = self.sn.backward(g.view(self.w.shape), self.w)
 
 
 class PointwiseNode:
@@ -142,7 +49,7 @@ class PointwiseNode:
         return w.view(w.shape[0], w.shape[1], 1, 1)
 
     def _pack(self, kindcode, rows_pad, cols_pad, planes, dtype=ops.BF16):
-        return _pack_generic(self.tape.cache, self.w, self._w4, "v111", kindcode, rows_pad, cols_pad, planes, dtype)
+        return pack_taps(self.tape.cache, self.w, self._w4, kindcode, rows_pad, cols_pad, planes, dtype)
 
     def _v(self, t, frames):
         return t.view(self.B, frames, self.x.H * self.x.W, t.shape[-1]) if t is not None else None
@@ -196,32 +103,11 @@ class VideoEncoderRunner:
     def apply(self, story):
         return TapeFn.apply(self, story, *[self.params[n] for n in self.names])[0]
 
-    # ---- stem conv (1, 7, 7): im2col GEMM
-    def _pack0(self, kind, planes=2, dtype=ops.BF16):
-        w = self.V.story_encoder[0][0].weight_orig
-        Co, K = w.shape[0], w.shape[1] * 49
-        Cop = rup(Co, 64)
-
-        def build():
-            w2 = w.detach().view(Co, w.shape[1], 7, 7).permute(0, 2, 3, 1).reshape(Co, K).contiguous()
-            if kind == "fwd":
-                t16 = ops.TORCH16[dtype]
-                hi = _e((Cop, STEM_K), w.device, t16)
-                lo = _e((Cop, STEM_K), w.device, t16) if planes == 2 else None
-                ops.pack_matrix(w2, Cop, STEM_K, K, K, 1, _row_pad_map(Co, Cop, w.device), hi, lo, dtype)
-                return [hi, lo]
-            hi = _e((STEM_K, Cop), w.device, torch.bfloat16)                        # [k, co]
-            ops.pack_matrix(w2, STEM_K, Cop, Co, 1, K, _row_pad_map(K, STEM_K, w.device), hi, None)
-            return hi
-        key = (id(w), "vstem_fwd", planes, dtype) if kind == "fwd" else (id(w), "vstem_bwd", 1, ops.BF16)
-        return _CACHE.get(key, w, build)
-
     def run_forward(self, story, *plist):
         V = self.V
         _eval_bn_unsupported(V)
         enc = V.story_encoder
         stem = enc[0]
-        dev = story.device
         B, Cin, T, H, W = story.shape
         assert Cin == 3 and H % 32 == 0 and W % 32 == 0, "VideoEncoder: 3-channel frames, sides multiple of 32"
         # hi/lo split operands also without grad: the logits of a no-grad call are the regression TARGET of the
@@ -236,21 +122,9 @@ class VideoEncoderRunner:
 
         # frames as batch entries: n = b * T + t
         frames = story.detach().permute(0, 2, 1, 3, 4).contiguous().view(B * T, Cin, H, W)
-        Ho, Wo = H // 2, W // 2
-        t16 = ops.TORCH16[tape.dtype]
-        col = T4(B * T, Ho, Wo, STEM_K)
-        col.hi = _e((B * T, Ho, Wo, STEM_K), dev, t16)
-        col.lo = _e((B * T, Ho, Wo, STEM_K), dev, t16) if tape.planes == 2 else None
-        ops.im2col_small(frames, 7, 2, 3, col.hi, col.lo, STEM_K, tape.dtype)
-        self.sn0, self.alpha0 = sn_of(stem[0])
-        Cop = rup(stem[0].weight_orig.shape[0], 64)
-        z0 = T4(B * T, Ho, Wo, Cop)
-        z0.f32 = _e((B * T, Ho, Wo, Cop), dev)
-        ops.conv_gemm(conv.gemm_nt([col.hi.view(-1, STEM_K), col.lo.view(-1, STEM_K) if col.lo is not None else None],
-                                   self._pack0("fwd", tape.planes, tape.dtype), z0.f32.view(-1, Cop),
-                                   alpha=self.alpha0, dtype=tape.dtype))
-        col.lo = None
-        self.col, self.z0 = col, z0
+        self.stem = Im2colNode(tape, frames, stem[0].weight_orig, "vstem.conv", 2, 3,
+                               sn=SpectralNorm(stem[0].weight_u, stem[0].weight_v))
+        z0 = tape.add(self.stem)
         bn0 = BnActNode(tape, z0, _bn_tuple(stem[1]), ops.ACT_RELU, "vstem.bn0")
         a = tape.add(bn0)
         sn, alpha = sn_of(stem[3])
@@ -263,9 +137,10 @@ class VideoEncoderRunner:
         for li, (idx, geom) in enumerate(LAYERS):
             sn, alpha = sn_of(enc[idx])
             if geom == "spatial":
-                cn = SpatialNode(tape, a, enc[idx].weight_orig, "venc%d" % idx, sn, alpha)
+                cn = ConvNode(tape, "s2k3", a, enc[idx].weight_orig, "venc%d" % idx, sn=sn, alpha=alpha,
+                              bn_stats=True)
             else:
-                cn = TemporalNode(tape, a, B, enc[idx].weight_orig, "venc%d" % idx, sn, alpha)
+                cn = TemporalNode(tape, a, B, enc[idx].weight_orig, "venc%d" % idx, 2, sn=sn, alpha=alpha)
             z = tape.add(cn)
             last = li == len(LAYERS) - 1
             bn = BnActNode(tape, z, _bn_tuple(enc[idx + 1]), ops.ACT_LRELU, "venc%d.bn" % idx, want_f32=last,
@@ -293,7 +168,6 @@ class VideoEncoderRunner:
         for nd in self.tape.nodes:
             if hasattr(nd, "x"):
                 nd.x.needs_grad = True
-        self.z0.needs_grad = True
         for cn, bn, idx in reversed(self.layers):
             bn.backward(need_w)
             pg["story_encoder.%d.weight" % (idx + 1)] = bn.dgamma
@@ -306,25 +180,13 @@ class VideoEncoderRunner:
         pw.backward(need_w)
         bn0.backward(need_w)
         pg["story_encoder.0.1.weight"], pg["story_encoder.0.1.bias"] = bn0.dgamma, bn0.dbeta
-        dz0 = self.z0.grad16
-        w0 = self.V.story_encoder[0][0].weight_orig
-        Co, Cop = w0.shape[0], self.z0.C
-        K = w0.shape[1] * 49
-        dz0m = dz0.view(-1, Cop)
-        if need_w:
-            d = _e((Cop, STEM_K), dev)
-            ops.conv_gemm(conv.gemm_tn(dz0m, self.col.hi.view(-1, STEM_K), d))
-            gw = d[:Co, :K].reshape(Co, 7, 7, w0.shape[1]).permute(0, 3, 1, 2).contiguous().view(w0.shape)
-            pg["story_encoder.0.0.weight_orig"] = self.sn0.backward(gw, w0)
+        dx = self.stem.backward(need_w, bool(needs[0]))
         dstory = None
-        if needs[0]:
+        if dx is not None:
             Bb, Cin, T, H, W = self.shape
-            dcol = _e((dz0m.shape[0], STEM_K), dev)
-            ops.conv_gemm(conv.gemm_nt([dz0m, None], [self._pack0("bwd"), None], dcol, alpha=self.alpha0))
-            dx = _e((Bb * T, Cin, H, W), dev)
-            ops.col2im_small(dcol, Bb * T, Cin, H, W, 7, 2, 3, dx)
             dstory = dx.view(Bb, T, Cin, H, W).permute(0, 2, 1, 3, 4)
         self.tape.aux.join()
+        pg["story_encoder.0.0.weight_orig"] = self.stem.dW
         pg["story_encoder.0.3.weight_orig"] = pw.dW
         for cn, _bn, idx in self.layers:
             pg["story_encoder.%d.weight_orig" % idx] = cn.dW
@@ -332,5 +194,5 @@ class VideoEncoderRunner:
         for nme, need in zip(self.names, needs[1:]):
             out.append(pg.get(nme) if need else None)
         self.tape.release()
-        self.tape = self.layers = self.stem_nodes = self.z0 = self.col = self.feat = None
+        self.tape = self.layers = self.stem_nodes = self.stem = self.feat = None
         return out

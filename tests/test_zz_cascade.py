@@ -1,7 +1,7 @@
 """Cascade generator (reference cascade_model.py; SURVEY.md section 8 row f2).
 
-Node level: the 3x3 / stride-2 downBlock convolution (run as the 4x4 / stride-2 implicit GEMM with
-zero 4th taps) and the 1-channel ``presample`` convolution (im2col GEMM), forward + dgrad + wgrad
+Node level: the 3x3 / stride-2 downBlock convolution (engine.ConvNode "s2k3": the 4x4 / stride-2 implicit
+GEMM with zero 4th taps) and the 1-channel ``presample`` convolution (engine.Im2colNode), forward + dgrad + wgrad
 against ``torch.nn.functional`` in fp64 -- on the CPU emulator of the kernel contract and,
 ``-m gpu``, on libcpcsv.so.  Step level (``-m gpu``): the whole cascade training step on the real
 kernels against the fp64 oracle and against the golden outputs of the REAL reference.
@@ -17,7 +17,7 @@ import torch.nn.functional as F
 
 import emulator
 import harness
-from cpcsv_b200 import cascade, engine, ops
+from cpcsv_b200 import engine, ops
 from oracle import presets
 from test_step_parity import (GOLD, _check, _check_against_golden, _check_generator_buffers, _step_pair)
 
@@ -56,16 +56,43 @@ def _planes_t4(x_nchw, cpad):
     return t
 
 
-@pytest.mark.parametrize("N,H,Ci,Co", [(3, 8, 60, 128), (2, 64, 2, 4), (5, 16, 64, 100)])
-def test_down_conv_node(dev, N, H, Ci, Co):
-    """conv3x3 stride 2 pad 1 (cascade_model.py:36-41) forward, data gradient, weight gradient"""
+def _sn(Co, K, dev):
+    """unit u [Co], v [K] of a spectral norm and an engine.SpectralNorm over copies of them"""
+    u = F.normalize(rnd(Co, seed=7), dim=0).to(dev)
+    v = F.normalize(rnd(K, seed=8), dim=0).to(dev)
+    return u.double(), v.double(), engine.SpectralNorm(u.clone(), v.clone())
+
+
+def _sigma(w, u, v):
+    """legacy torch spectral_norm in fp64: one power iteration from (u, v), then sigma = u^T W v, differentiable
+    in w with the iterated u, v held constant"""
+    w2 = w.reshape(w.shape[0], -1)
+    with torch.no_grad():
+        v = F.normalize(w2.t() @ u, dim=0, eps=1e-12)
+        u = F.normalize(w2 @ v, dim=0, eps=1e-12)
+    return u @ (w2 @ v)
+
+
+@pytest.mark.parametrize("N,H,Ci,Co,sn", [(3, 8, 60, 128, False), (2, 64, 2, 4, False), (5, 16, 64, 100, False),
+                                          # Conv3d (1, 3, 3) weight with a spectral norm (the video critic's layers)
+                                          (2, 16, 24, 40, True)])
+def test_s2k3_conv_node(dev, N, H, Ci, Co, sn):
+    """conv3x3 stride 2 pad 1 (cascade_model.py:36-41) as engine.ConvNode's "s2k3" geometry: forward, data
+    gradient, weight gradient"""
     x = rnd(N, Ci, H, H, seed=1, dev=dev)
-    w = torch.nn.Parameter(rnd(Co, Ci, 3, 3, seed=2, dev=dev, scale=0.05))
+    shape = (Co, Ci, 1, 3, 3) if sn else (Co, Ci, 3, 3)
+    w = torch.nn.Parameter(rnd(*shape, seed=2, dev=dev, scale=0.05))
     tape = engine.Tape(engine.WeightCache(), training=True, need_grad=True)
     a = _planes_t4(x, engine.rup(Ci, 64))
-    node = cascade.DownConvNode(tape, a, w, "down")
+    u, v, snm = _sn(Co, Ci * 9, dev) if sn else (None, None, None)
+
+    def w_eff(wd, wsig):
+        """the 4-D weight the convolution applies; wsig: the weight sigma is computed from"""
+        w4 = wd.view(Co, Ci, 3, 3)
+        return w4 / _sigma(wsig, u, v) if sn else w4
+    node = engine.ConvNode(tape, "s2k3", a, w, "down", sn=snm)
     out = tape.add(node)
-    ref = F.conv2d(x.double(), w.detach().double(), stride=2, padding=1)
+    ref = F.conv2d(x.double(), w_eff(w.detach().double(), w.detach().double()), stride=2, padding=1)
     got = out.f32.permute(0, 3, 1, 2)
     assert rel(got[:, :Co], ref) < 3e-5
     assert got.shape[1] == Co or float(got[:, Co:].abs().max()) == 0.0
@@ -77,42 +104,53 @@ def test_down_conv_node(dev, N, H, Ci, Co):
     node.backward(True)
     tape.aux.join()
     xd = bf16r(x).double().requires_grad_(True)
-    wd = bf16r(w.detach()).double().requires_grad_(True)
-    y = F.conv2d(xd, wd, stride=2, padding=1)
+    wd = w.detach().double().requires_grad_(True)
     dzr = bf16r(dz)[..., :Co].permute(0, 3, 1, 2).double()
-    gx, _ = torch.autograd.grad(y, (xd, wd), dzr, retain_graph=True)
+    y = F.conv2d(xd, w_eff(bf16r(w.detach()).double(), w.detach().double()), stride=2, padding=1)
+    gx = torch.autograd.grad(y, xd, dzr)[0]
     assert rel(a.grad.permute(0, 3, 1, 2)[:, :Ci], gx) < 1e-5
-    gw = torch.autograd.grad(F.conv2d(bf16r(x).double(), wd, stride=2, padding=1), wd, dzr)[0]
-    assert tuple(node.dW.shape) == (Co, Ci, 3, 3)
+    gw = torch.autograd.grad(F.conv2d(bf16r(x).double(), w_eff(wd, wd), stride=2, padding=1), wd, dzr)[0]
+    assert tuple(node.dW.shape) == shape
     assert rel(node.dW, gw) < 1e-5
 
 
 @pytest.mark.parametrize("planes,dtype", [(2, ops.BF16), (1, ops.FP16)])
-@pytest.mark.parametrize("N,Co", [(3, 2), (2, 64)])
-def test_mask_conv(dev, planes, dtype, N, Co):
-    """presample's conv3x3(1 -> Co) on the 1-channel mask (cascade_model.py:312-316)"""
-    x = torch.tanh(rnd(N, 1, 64, 64, seed=4, dev=dev))
-    w = torch.nn.Parameter(rnd(Co, 1, 3, 3, seed=5, dev=dev, scale=0.3))
+@pytest.mark.parametrize("N,Co,k,stride,pad,Ci,sn", [(3, 2, 3, 1, 1, 1, False), (2, 64, 3, 1, 1, 1, False),
+                                                     # the video critic's stem: (1, 7, 7) stride (1, 2, 2)
+                                                     # pad (0, 3, 3) on 3 channels with a spectral norm
+                                                     (2, 16, 7, 2, 3, 3, True)])
+def test_im2col_node(dev, planes, dtype, N, Co, k, stride, pad, Ci, sn):
+    """engine.Im2colNode: presample's conv3x3(1 -> Co) on the 1-channel mask (cascade_model.py:312-316), and a
+    spectrally normalised 7x7 stride-2 convolution with K = 147 -> 192"""
+    x = torch.tanh(rnd(N, Ci, 64, 64, seed=4, dev=dev))
+    w = torch.nn.Parameter(rnd(Co, Ci, k, k, seed=5, dev=dev, scale=0.3))
     need_grad = planes == 2
     tape = engine.Tape(engine.WeightCache(), training=True, need_grad=need_grad, planes=planes, dtype=dtype)
-    mc = cascade.MaskConv(tape, w, "presample")
-    z = mc.forward(x)
-    ref = F.conv2d(x.double(), w.detach().double(), padding=1)
+    u, v, snm = _sn(Co, Ci * k * k, dev) if sn else (None, None, None)
+
+    def w_eff(wd, wsig):
+        return wd / _sigma(wsig, u, v) if sn else wd
+    mc = engine.Im2colNode(tape, x, w, "presample", stride, pad, sn=snm)
+    z = tape.add(mc)
+    ref = F.conv2d(x.double(), w_eff(w.detach().double(), w.detach().double()), stride=stride, padding=pad)
     got = z.f32.permute(0, 3, 1, 2)
     assert rel(got[:, :Co], ref) < (3e-5 if planes == 2 else 1e-3)
     assert got.shape[1] == Co or float(got[:, Co:].abs().max()) == 0.0
     if not need_grad:
         return
-    dz = torch.zeros(N, 64, 64, z.C, device=dev)
-    dz[..., :Co] = rnd(N, 64, 64, Co, seed=6, dev=dev)
+    Ho = 64 // stride
+    dz = torch.zeros(N, Ho, Ho, z.C, device=dev)
+    dz[..., :Co] = rnd(N, Ho, Ho, Co, seed=6, dev=dev)
     z.grad16 = dz.to(torch.bfloat16)
     dx = mc.backward(True, True)
     tape.aux.join()
     xd = bf16r(x).double().requires_grad_(True)
-    wd = bf16r(w.detach()).double().requires_grad_(True)
+    wd = w.detach().double().requires_grad_(True)
     dzr = bf16r(dz)[..., :Co].permute(0, 3, 1, 2).double()
-    assert rel(mc.dW, torch.autograd.grad(F.conv2d(xd.detach(), wd, padding=1), wd, dzr)[0]) < 1e-5
-    gxr = torch.autograd.grad(F.conv2d(xd, wd.detach(), padding=1), xd, dzr)[0]
+    gw = torch.autograd.grad(F.conv2d(xd.detach(), w_eff(wd, wd), stride=stride, padding=pad), wd, dzr)[0]
+    assert rel(mc.dW, gw) < 1e-5
+    wb = w_eff(bf16r(w.detach()).double(), w.detach().double())
+    gxr = torch.autograd.grad(F.conv2d(xd, wb, stride=stride, padding=pad), xd, dzr)[0]
     assert rel(dx, gxr) < 1e-5
 
 
