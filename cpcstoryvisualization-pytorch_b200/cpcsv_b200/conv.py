@@ -19,14 +19,35 @@ NUM_SMS = 148
 def pixel_tile(N, H, W, rows):
     """Box (tile_n, tile_h, tile_w) of `rows` pixels.  W is a power of two; H usually is -- for any other H (an odd
     number of frames of the temporal convolutions) the box height is the next power of two: the kernel masks rows
-    outside the grid and TMA zero-fills their loads."""
+    outside the grid and TMA zero-fills their loads.  A grid this rule cannot tile (a W that is no power of two,
+    the 147 / 73 / 35 / 17 grids of InceptionV3) gets the box with the fewest masked rows (_min_waste_tile)."""
     tw = min(W, rows)
     th = 1
     while th < H and th * 2 <= rows // tw:
         th *= 2
     tn = rows // (tw * th)
-    assert tn * th * tw == rows, (N, H, W, rows)
+    if tn * th * tw != rows:
+        return _min_waste_tile(N, H, W, rows)
     return tn, th, tw
+
+
+def _min_waste_tile(N, H, W, rows):
+    """the power-of-two box of `rows` pixels whose tiles cover the (N, H, W) grid with the fewest masked rows; ties
+    go to the wider, then the taller box.  Any such box is legal: every pixel row of the A tile is one 128-B
+    channel segment whatever the box shape, and the epilogue masks rows outside the grid."""
+    best = None
+    tw = 1
+    while tw <= rows:
+        th = 1
+        while tw * th <= rows:
+            tn = rows // (tw * th)
+            cover = -(-N // tn) * tn * (-(-H // th) * th) * (-(-W // tw) * tw)
+            key = (cover, -tw, -th)
+            if best is None or key < best[0]:
+                best = (key, (tn, th, tw))
+            th *= 2
+        tw *= 2
+    return best[1]
 
 
 def pick_block_n(npad):
@@ -76,15 +97,20 @@ def _m_tiles(grid, tile):
 
 
 def _fwd_job(a_planes, b_planes, grid, groups, taps_per_group, taps, k_blocks, out, npad,
-             out_strides, alpha=None, accumulate=False, dtype=BF16, splits=None):
+             out_strides, alpha=None, accumulate=False, dtype=BF16, splits=None, n_valid=None):
+    """`npad`: weight rows per tap (the N extent of the GEMM); `n_valid`: output columns stored (default npad), less
+    when the output is a channel slice of a wider buffer"""
     tile = pixel_tile(*grid, 128)
     block_n = pick_block_n(npad)
     n_tiles = npad // block_n
+    if n_valid is None:
+        n_valid = npad
+    assert n_valid <= npad, (n_valid, npad)
     if splits is None:
         splits = pick_splits(groups * _m_tiles(grid, tile) * n_tiles, taps_per_group * k_blocks)
     return GemmJob(mode=0, planes=len(a_planes), grid=grid, tile=tile, groups=groups,
                    taps_per_group=taps_per_group, k_blocks=k_blocks, taps=taps, a=a_planes,
-                   b=b_planes, out=out, n_valid=npad, block_n=block_n, n_tiles=n_tiles,
+                   b=b_planes, out=out, n_valid=n_valid, block_n=block_n, n_tiles=n_tiles,
                    splits=splits, accumulate=accumulate, out_strides=out_strides, alpha=alpha,
                    dtype=dtype, pair=use_pair(grid, tile, block_n))
 
@@ -356,3 +382,51 @@ def conv_t3_wgrad(dy, x_hi, dwt):
         taps = [((0, 0, 0, 0), (0, 0, 0, -1), 0 * Co * Ci), ((0, 0, 0, 0), (0, 0, 0, 0), 2 * Co * Ci)]
         jobs.append(_wgrad_job(View.nhwc(dy), View.nhwc(xo), (B, To, HW), taps, Co, Ci, dwt, Ci, accumulate=True))
     return jobs
+
+
+# ------------------------------------------------------------------ InceptionV3 geometries (frame FID)
+def conv_kxl_fwd(x_planes, w_planes, out, kh, kw, ph, pw, dtype=BF16, splits=None):
+    """out[N, Ho, Wo, :n] = conv(x[N, H, W, Ci], w), stride 1, kernel kh x kw, padding (ph, pw): Ho = H + 2 ph - kh + 1
+    (smaller than H for an unpadded 3x3).  Tap (ky, kx) reads x[h + ky - ph, w + kx - pw]; TMA's zero fill outside
+    the view is the padding.  w_planes: packed kind 0 ``[kh*kw * Co_pad, Ci]`` (tap ky*kw + kx at rows
+    [tap * Co_pad, ...)).  ``out`` may be a channel slice ``buf[..., c0:c0 + n]`` of a wider fp32 buffer (c0 and
+    the pitches multiples of 4): n <= Co_pad columns are stored.  More than CPCSV_MAX_TAPS = 16 taps (5x5) run as
+    two jobs on the same output: the first 16 taps overwrite, the rest add with one red.add per element
+    (``splits`` 1 for both), so the result stays bit-reproducible.  Returns the list of jobs."""
+    N, H, W, Ci = x_planes[0].shape
+    Ho, Wo = H + 2 * ph - kh + 1, W + 2 * pw - kw + 1
+    assert tuple(out.shape[:3]) == (N, Ho, Wo), (tuple(out.shape), (N, Ho, Wo))
+    ntap = kh * kw
+    npad = w_planes[0].shape[0] // ntap
+    assert npad * ntap == w_planes[0].shape[0] and npad % 64 == 0
+    taps = [((0, kx - pw, 0, ky - ph), ((ky * kw + kx) * npad, 0, 0, 0), 0) for ky in range(kh) for kx in range(kw)]
+    chunks = [taps[i:i + 16] for i in range(0, ntap, 16)]
+    if len(chunks) > 1:
+        splits = 1
+    av, bv = _planes(x_planes, View.nhwc), _planes(w_planes, View.matrix)
+    return [_fwd_job(av, bv, (N, Ho, Wo), 1, len(ch), ch, Ci // 64, out, npad, _plain_out_strides(out),
+                     accumulate=i > 0, dtype=dtype, splits=splits, n_valid=out.shape[-1])
+            for i, ch in enumerate(chunks)]
+
+
+def conv_s2v_fwd(x_planes, w_planes, out, dtype=BF16, splits=None):
+    """out[N, So, So, :n] = conv3x3 stride 2 pad 0 (x), So = (S - 3) // 2 + 1, as one 9-tap job on the parity view:
+    tap k of a row / column reads parity k % 2 at block offset k // 2 (input index 2 o + k).
+
+    Layout of an odd-sized input (S = 35, 17): ``x_planes`` are the WHOLE buffers ``[N, S + 1, S + 1, Ci]``, one
+    extra row and column that a valid output never reads (its largest index is 2 (So - 1) + 2 = S - 1), so
+    ``View.nhwc_parity`` applies to them; stride-1 consumers of the same activation read the ``[:, :S, :S]``
+    slice, whose view dims are S, so TMA zero-fills exactly the padding.  Rows of the pixel box beyond the output
+    grid may read the extra row / column; the kernel masks them.  Even S needs no extra row.
+    w_planes: kind 0 ``[9 * Co_pad, Ci]``; ``out`` may be a channel slice as in conv_kxl_fwd."""
+    N, P, P2, Ci = x_planes[0].shape
+    So = out.shape[1]
+    assert P == P2 and P % 2 == 0 and out.shape[2] == So and 2 * So + 1 <= P, (tuple(x_planes[0].shape), So)
+    npad = w_planes[0].shape[0] // 9
+    assert npad * 9 == w_planes[0].shape[0] and npad % 64 == 0
+    taps = []
+    for ky in range(3):
+        for kx in range(3):
+            taps.append((((kx % 2) * Ci, kx // 2, ky % 2, ky // 2), ((ky * 3 + kx) * npad, 0, 0, 0), 0))
+    return _fwd_job(_planes(x_planes, View.nhwc_parity), _planes(w_planes, View.matrix), (N, So, So), 1, 9, taps,
+                    Ci // 64, out, npad, _plain_out_strides(out), dtype=dtype, splits=splits, n_valid=out.shape[-1])

@@ -715,8 +715,9 @@ class BnActNode:
     """[BatchNorm (batch statistics)] -> activation -> [* (1 + mod)] -> operand planes / fp32."""
 
     def __init__(self, tape, z, bn, act, name, mod=None, want_f32=False, want_planes=True,
-                 chan_map=None, c_valid=None, pre_bias=None):
+                 chan_map=None, c_valid=None, pre_bias=None, eps=1e-5):
         self.tape, self.z, self.bn, self.act, self.name, self.mod = tape, z, bn, act, name, mod
+        self.eps = eps      # of the eval-mode normalisation (InceptionV3's BasicConv2d: 1e-3)
         # bias of the producing conv that was NOT added to z (a batch-statistics BatchNorm removes it;
         # only the eval-mode normalisation with running statistics has to account for it)
         self.pre_bias = pre_bias
@@ -747,7 +748,7 @@ class BnActNode:
             if t.need_grad:
                 raise NotImplementedError("cpcsv_b200: backward through eval-mode BatchNorm is not implemented "
                                           "(the reference only evaluates under torch.no_grad())")
-            scale, shift = eval_affine(self.bn, z.C, self.chan_map, self.c_valid)
+            scale, shift = eval_affine(self.bn, z.C, self.chan_map, self.c_valid, self.eps)
             if self.pre_bias is not None:
                 b = torch.zeros(z.C, device=dev)
                 b[:self.pre_bias.numel()].copy_(self.pre_bias.detach())

@@ -220,6 +220,43 @@ def bn_norm_act_pack(x, stats, gamma, beta, running_mean, running_var, chan_map,
         ldp, dtype, _stream()), "cpcsv_bn_norm_act_pack")
 
 
+# ------------------------------------------------------------------ frame FID (InceptionV3)
+POOL_MAX, POOL_AVG = 0, 1
+
+
+def resize_im2col(x, S, a, b, hi, lo, dtype=BF16):
+    """x fp32 [N, 3, H, W] (any strides) -> im2col rows [N * OH * OH, ldp] of the 3x3 stride-2 pad-0 conv on the
+    bilinear S x S resize of a * x + b, OH = (S - 3) // 2 + 1 (include/cpcsv.h cpcsv_resize_im2col)"""
+    N, Cc, H, W = x.shape
+    assert Cc == 3
+    ldp = hi.shape[-1]
+    OH = (S - 3) // 2 + 1
+    assert hi.is_contiguous() and hi.numel() == N * OH * OH * ldp
+    assert lo is None or (lo.is_contiguous() and lo.shape == hi.shape)
+    sn, sc, sh, sw = x.stride()
+    _lib.check(_lib.load().cpcsv_resize_im2col(
+        _ptr(x, torch.float32), N, H, W, sn, sc, sh, sw, S, float(a), float(b), _ptr(hi, TORCH16[dtype]),
+        _ptr(lo, TORCH16[dtype]), ldp, dtype, _stream()), "cpcsv_resize_im2col")
+
+
+def pool3x3(x, mode, stride, y=None, hi=None, lo=None, dtype=BF16):
+    """3x3 max (POOL_MAX) / average without the padding (POOL_AVG) pooling, stride 1 pad 1 or stride 2 pad 0, of
+    x fp32 [N, H, W, C] (channels contiguous, any pixel pitches) into fp32 y and / or 16-bit hi / lo planes
+    [N, Ho, Wo, C] (channel slices of wider buffers allowed)"""
+    N, H, W, Cc = x.shape
+    Ho = H if stride == 1 else (H - 3) // 2 + 1
+    Wo = W if stride == 1 else (W - 3) // 2 + 1
+    for t in (y, hi, lo):
+        assert t is None or (tuple(t.shape) == (N, Ho, Wo, Cc) and t.stride(3) == 1), (None if t is None else t.shape)
+    assert x.stride(3) == 1 and (lo is None or lo.stride() == hi.stride())
+    ys = y.stride()[:3] if y is not None else (0, 0, 0)
+    ps = hi.stride()[:3] if hi is not None else (0, 0, 0)
+    _lib.check(_lib.load().cpcsv_pool3x3(
+        _ptr(x, torch.float32), N, H, W, Cc, x.stride(0), x.stride(1), x.stride(2), mode, stride,
+        _ptr(y, torch.float32), ys[0], ys[1], ys[2], _ptr(hi, TORCH16[dtype]), _ptr(lo, TORCH16[dtype]), ps[0],
+        ps[1], ps[2], dtype, _stream()), "cpcsv_pool3x3")
+
+
 # ------------------------------------------------------------------ layout kernels
 def images_to_u8(x, out):
     """x [C, H, W] fp32 in [-1, 1] (any strides) -> out uint8 [H, W, C] (contiguous)"""

@@ -764,10 +764,45 @@ class GANTrainer(object):
         generator's noise is drawn from a generator seeded with ``seed`` (the global RNG state is restored
         afterwards), so the value is reproducible.  ``netG`` is left in train mode."""
         from cpcsv_b200 import fsd
-        dev = next(netG.parameters()).device
-        text_dim = cfg.TEXT.DIMENSION
         real = fsd.FeatureStats() if real_stats is None else None
         fake = fsd.FeatureStats()
+        for fake_stories, real_stories in self._sample_test_stories(netG, testloader, seed):
+            fake.update(feature_net(fake_stories))
+            if real is not None:
+                real.update(feature_net(real_stories))
+        real = real if real is not None else real_stats
+        value = fsd.frechet_distance(real.mu, real.sigma, fake.mu.to(real.mu.device), fake.sigma.to(real.mu.device))
+        if self._logger is not None:
+            self._logger.add_scalar("Evaluation/fsd", value, epoch)
+        return value
+
+    def calculate_fid(self, netG, testloader, feature_net, real_stats=None, epoch=None, seed=0):
+        """Frame-level FID of generated test stories on the kernel path (cpcsv_b200.frame_fid), the frame
+        counterpart of ``calculate_fsd``: InceptionV3 pool3 features (``feature_net``, a
+        ``frame_fid.FrameFeatureNet``) of every frame of the real ``images`` of every test batch and of every frame
+        the generator produces for the same batch (eval mode, no_grad, noise seeded with ``seed``, the RNG state
+        restored, ``netG`` left in train mode).  ``real_stats``: a ``fsd.FeatureStats(dim=2048)`` of the real
+        frames computed (``frame_fid.frame_statistics``) or loaded before.  Logged as ``Evaluation/frame_fid``;
+        ``calculate_vfid`` (the reference's ``fid/`` package) is unchanged."""
+        from cpcsv_b200 import frame_fid, fsd
+        real = fsd.FeatureStats(dim=frame_fid.FEATURE_DIM) if real_stats is None else None
+        fake = fsd.FeatureStats(dim=frame_fid.FEATURE_DIM)
+        for fake_stories, real_stories in self._sample_test_stories(netG, testloader, seed):
+            frame_fid.frame_statistics([fake_stories], feature_net, fake)
+            if real is not None:
+                frame_fid.frame_statistics([real_stories], feature_net, real)
+        real = real if real is not None else real_stats
+        value = fsd.frechet_distance(real.mu, real.sigma, fake.mu.to(real.mu.device), fake.sigma.to(real.mu.device))
+        if self._logger is not None:
+            self._logger.add_scalar("Evaluation/frame_fid", value, epoch)
+        return value
+
+    def _sample_test_stories(self, netG, testloader, seed):
+        """yields (generated stories, real ``images``) of every test batch: ``netG.sample_videos`` in eval mode under
+        no_grad, with noise from a generator seeded with ``seed``; the global RNG state is restored and ``netG``
+        is back in train mode once the loop ends"""
+        dev = next(netG.parameters()).device
+        text_dim = cfg.TEXT.DIMENSION
         netG.eval()
         try:
             with torch.no_grad(), torch.random.fork_rng(devices=[dev] if dev.type == "cuda" else []):
@@ -777,16 +812,9 @@ class GANTrainer(object):
                     st_content = description[:, :, :text_dim]
                     st_motion = torch.cat((st_content, batch["labels"].to(dev)), 2)
                     _, fake_stories, _, _, _, _, _ = netG.sample_videos(st_motion, st_content)
-                    fake.update(feature_net(fake_stories))
-                    if real is not None:
-                        real.update(feature_net(batch["images"].to(dev)))
+                    yield fake_stories, batch["images"].to(dev)
         finally:
             netG.train()
-        real = real if real is not None else real_stats
-        value = fsd.frechet_distance(real.mu, real.sigma, fake.mu.to(real.mu.device), fake.sigma.to(real.mu.device))
-        if self._logger is not None:
-            self._logger.add_scalar("Evaluation/fsd", value, epoch)
-        return value
 
     GRAPH_WARMUP_STEPS = 3      # eager steps (optimiser state, weight caches, NCCL) before the capture
 

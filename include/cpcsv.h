@@ -165,6 +165,25 @@ int cpcsv_bn_add_act_pack(const float* x, int64_t rows, int32_t C, int64_t ldx, 
                           const float* rshift, int32_t act, float* y, int64_t ldy, void* hi, void* lo,
                           int64_t ldp, int32_t dtype, cpcsv_stream_t stream);
 
+/* ------------------------------------------------------------------- frame FID (InceptionV3) */
+/* Stem input of the FID InceptionV3 (cpcsv_b200/frame_fid.py): the fp32 NCHW 3-channel frames x [N, 3, H, W]
+ * (element strides sn, sc, sh, sw, any size) resized bilinearly to S x S (align_corners=False, no antialias,
+ * PyTorch's source-index rule), mapped by v = a * sample + b, and written as the im2col rows of the 3x3 stride-2
+ * pad-0 Conv2d_1a_3x3: row (n, oh, ow) of OH = (S - 3) / 2 + 1, column (ky*3 + kx)*3 + c (< 27; columns up to ldp
+ * are zero), as 16-bit hi / lo (lo optional) planes with row pitch ldp (a multiple of 8, 16-B aligned planes).
+ * The S x S image is never materialised. */
+int cpcsv_resize_im2col(const float* x, int32_t N, int32_t H, int32_t W, int64_t sn, int64_t sc, int64_t sh,
+                        int64_t sw, int32_t S, float a, float b, void* hi, void* lo, int32_t ldp, int32_t dtype,
+                        cpcsv_stream_t stream);
+/* 3x3 pooling of a pitched fp32 NHWC input x [N, H, W, C] (pixel pitches sn, sh, sw in elements, channels
+ * contiguous, C % 4 == 0): mode 0 max, mode 1 average over the taps inside the input (count_include_pad=False);
+ * stride 1 pad 1 (output H x W) or stride 2 pad 0 (output (H - 3) / 2 + 1).  Writes fp32 y (a channel slice of
+ * a wider buffer: pitches ysn, ysh, ysw) and / or 16-bit hi / lo planes (pitches psn, psh, psw); all pitches
+ * multiples of 4 elements, x / y 16-B and the planes 8-B aligned. */
+int cpcsv_pool3x3(const float* x, int32_t N, int32_t H, int32_t W, int32_t C, int64_t sn, int64_t sh, int64_t sw,
+                  int32_t mode, int32_t stride, float* y, int64_t ysn, int64_t ysh, int64_t ysw, void* hi, void* lo,
+                  int64_t psn, int64_t psh, int64_t psw, int32_t dtype, cpcsv_stream_t stream);
+
 /* ------------------------------------------------------------------- layout / pack kernels */
 /* generated frames / image sheets for the PNG writers (miscc/utils.py:230-235 images_to_numpy,
  * inference.py:181-197): x [C, H, W] fp32 in [-1, 1] with element strides (sc, sh, sw) ->
