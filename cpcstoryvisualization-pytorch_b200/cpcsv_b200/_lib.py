@@ -71,6 +71,8 @@ SIGNATURES = {
     "cpcsv_resize_im2col": [_p, _i32, _i32, _i32, _i64, _i64, _i64, _i64, _i32, _f32, _f32, _p, _p, _i32, _i32, _p],
     "cpcsv_pool3x3": [_p, _i32, _i32, _i32, _i32, _i64, _i64, _i64, _i32, _i32, _p, _i64, _i64, _i64, _p, _p, _i64,
                       _i64, _i64, _i32, _p],
+    "cpcsv_ssim": [_p, _p, _i32, _i32, _i32, _i32, _i32, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i64, _i64,
+                   _f32, _f32, _p, _p],
     "cpcsv_images_to_u8": [_p, _i32, _i32, _i32, _i64, _i64, _i64, _p, _p],
     "cpcsv_pack_nchw": [_p, _i32, _i32, _i32, _i32, _i64, _i64, _i64, _i64, _p, _i32, _i64, _p, _p,
                         _i32, _i32, _p],

@@ -257,6 +257,18 @@ def pool3x3(x, mode, stride, y=None, hi=None, lo=None, dtype=BF16):
         ps[1], ps[2], dtype, _stream()), "cpcsv_pool3x3")
 
 
+# ------------------------------------------------------------------ frame SSIM
+def ssim(x, y, a, b, out):
+    """out fp64 [B * T] = per-frame SSIM of a * x + b against a * y + b; x, y fp32 [B, T, C, H, W] of the same shape,
+    any strides (include/cpcsv.h cpcsv_ssim)"""
+    B, T, Cc, H, W = x.shape
+    assert tuple(y.shape) == tuple(x.shape), (x.shape, y.shape)
+    assert out.is_contiguous() and out.numel() == B * T, (out.shape, B * T)
+    _lib.check(_lib.load().cpcsv_ssim(
+        _ptr(x, torch.float32), _ptr(y, torch.float32), B, T, Cc, H, W, *x.stride(), *y.stride(), float(a), float(b),
+        _ptr(out, torch.float64), _stream()), "cpcsv_ssim")
+
+
 # ------------------------------------------------------------------ layout kernels
 def images_to_u8(x, out):
     """x [C, H, W] fp32 in [-1, 1] (any strides) -> out uint8 [H, W, C] (contiguous)"""

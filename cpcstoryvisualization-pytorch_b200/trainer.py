@@ -797,6 +797,20 @@ class GANTrainer(object):
             self._logger.add_scalar("Evaluation/frame_fid", value, epoch)
         return value
 
+    def calculate_ssim(self, netG, testloader, epoch=None, seed=0):
+        """Mean SSIM of generated test stories on the kernel path (cpcsv_b200.ssim), the SSIM counterpart of
+        ``calculate_fsd`` (reference trainer.py:175-182, through ``pytorch_ssim``): over every frame of every test
+        batch, between the story the generator produces for the batch (eval mode, no_grad, noise seeded with
+        ``seed``, the RNG state restored, ``netG`` left in train mode) and the batch's real ``images``.  Both are in
+        [-1, 1], mapped to [0, 1] inside the kernel.  Logged as ``Evaluation/ssim``."""
+        from cpcsv_b200 import ssim
+        scores = [ssim.frame_ssim(fake_stories, real_stories, input_range=(-1, 1))
+                  for fake_stories, real_stories in self._sample_test_stories(netG, testloader, seed)]
+        value = float(torch.cat(scores).mean())
+        if self._logger is not None:
+            self._logger.add_scalar("Evaluation/ssim", value, epoch)
+        return value
+
     def _sample_test_stories(self, netG, testloader, seed):
         """yields (generated stories, real ``images``) of every test batch: ``netG.sample_videos`` in eval mode under
         no_grad, with noise from a generator seeded with ``seed``; the global RNG state is restored and ``netG``

@@ -184,6 +184,21 @@ int cpcsv_pool3x3(const float* x, int32_t N, int32_t H, int32_t W, int32_t C, in
                   int32_t mode, int32_t stride, float* y, int64_t ysn, int64_t ysh, int64_t ysw, void* hi, void* lo,
                   int64_t psn, int64_t psh, int64_t psw, int32_t dtype, cpcsv_stream_t stream);
 
+/* ------------------------------------------------------------------- frame SSIM */
+/* Per-frame SSIM of the reference's evaluation (ssim_score.py / the SSIM loop of trainer.py:175-182, which call
+ * pytorch_ssim.ssim(x, y, size_average=False)): x, y fp32 with logical layout [B, T, C, H, W] and element strides
+ * (xsb, xst, xsc, xsh, xsw) / (ysb, ...) -- stories [B, C, T, H, W] without a copy, plain frames as T = 1 -- both
+ * mapped by v = a * v + b on load.  out[b * T + t] (fp64) = the mean over C x H x W of the SSIM map of frame (b, t):
+ * 11-tap Gaussian window (sigma 1.5, sum 1) per channel, zero padding 5 (border windows see zeros, no
+ * renormalisation), sigma^2 = E[v^2] - mu^2, sigma_xy = E[xy] - mu_x mu_y, C1 = 0.01^2, C2 = 0.03^2,
+ * ssim = ((2 mu_x mu_y + C1)(2 sigma_xy + C2)) / ((mu_x^2 + mu_y^2 + C1)(sigma_x^2 + sigma_y^2 + C2)).
+ * Moments in fp32, the mean in fp64.  Any C, H, W >= 1.  One CTA per frame, no atomics: a frame's value depends
+ * only on its own pixels (not on B, its index or the other frames) and is bit-reproducible. */
+int cpcsv_ssim(const float* x, const float* y, int32_t B, int32_t T, int32_t C, int32_t H, int32_t W,
+               int64_t xsb, int64_t xst, int64_t xsc, int64_t xsh, int64_t xsw,
+               int64_t ysb, int64_t yst, int64_t ysc, int64_t ysh, int64_t ysw,
+               float a, float b, double* out, cpcsv_stream_t stream);
+
 /* ------------------------------------------------------------------- layout / pack kernels */
 /* generated frames / image sheets for the PNG writers (miscc/utils.py:230-235 images_to_numpy,
  * inference.py:181-197): x [C, H, W] fp32 in [-1, 1] with element strides (sc, sh, sw) ->
